@@ -5,6 +5,8 @@
   python bench.py --impl reference [...]                    reference arm: the CPU implementation
                                                             (oracle port of nnnoiseless 0.5.2; the
                                                             crate itself cannot be built offline)
+  python bench.py [...] --dump-outputs DIR                  also write the last timed step's outputs (a seeded
+                                                            sample of frames) as DIR/<name>.npy
 
 A "step" is one pass of the whole denoise path over one batch: configs[1] of BASELINE.json --
 1,024 independent 60 s 48 kHz mono streams per GPU (6.144 M frames), synthetic speech+noise.
@@ -35,6 +37,8 @@ PITCH_MACS_PER_FRAME = 75000        # K1: multiply-adds per frame that must stay
 FP32_PEAK_TFLOPS_NOMINAL = 74.5     # 148 SM * 128 lanes * 2 * 1.965 GHz (not in MEASURED_PEAKS.json)
 # the recurrent core (K4) runs on the tensor pipe: 723 bf16 m16n8k16 tiles per 16-stream step, twice (hi + lo plane)
 RNN_MMA_FLOPS_PER_FRAME = 2 * 723 * (16 * 8 * 16 * 2) // 16   # executed flops per (stream, frame), padding included
+# frames per array --dump-outputs writes: 8,192 x (960 + 1) x 4 B = 31.5 MB for the widest step (c4's stereo mix + VAD)
+DUMP_FRAMES = 8192
 
 
 def parse_args():
@@ -58,7 +62,32 @@ def parse_args():
     ap.add_argument("--total-streams", type=int, default=None, help="c4/c5: streams (meetings) in the whole job")
     ap.add_argument("--minutes", type=float, default=None, help="c4/c5: recording length (default 10 / 60)")
     ap.add_argument("--chunk-seconds", type=int, default=10, help="c4/c5: audio seconds per call")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what rank 0's last timed step returned (the denoised audio and "
+                         "the VAD; c3-c5: of the step's last call) as DIR/<name>.npy, float32, sampled to "
+                         f"{DUMP_FRAMES} frames by a fixed seed, so that two builds can be compared output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU path's outputs; the reference arm has none to write")
+    return args
+
+
+def dump_outputs(dump_dir: str, n_frames: int, arrays: dict) -> None:
+    """Writes each [streams, frames x k] output as DIR/<name>.npy, float32 [DUMP_FRAMES, k] (k = 1 is squeezed): the
+    frames at the same (stream, frame) pairs, drawn without replacement by numpy's default_rng(0) and sorted, in every
+    array and every run."""
+    import numpy as np
+    import torch
+    n_streams = next(iter(arrays.values())).shape[0]
+    total = n_streams * n_frames
+    pick = torch.from_numpy(np.sort(np.random.default_rng(0).choice(total, min(DUMP_FRAMES, total), replace=False)))
+    os.makedirs(dump_dir, exist_ok=True)
+    for name, a in arrays.items():
+        s, f = (pick // n_frames).to(a.device), (pick % n_frames).to(a.device)
+        sample = a.reshape(n_streams, n_frames, -1)[s, f].squeeze(-1)
+        np.save(os.path.join(dump_dir, name + ".npy"), sample.float().cpu().numpy())
 
 
 def measured_peaks():
@@ -338,6 +367,8 @@ def run_b200(args):
     clocks = sampler.stop() if rank == 0 else None
     total_ms = evs[0][0].elapsed_time(evs[-1][1])
     launches = den.info["launches"] - launches0
+    if rank == 0 and args.dump_outputs:  # before the profiled step and the serial leg below write into out / vad
+        dump_outputs(args.dump_outputs, n_frames, {"out": out, "vad": vad})
     # per-kernel launch durations: one more step of the same workload, OUTSIDE the timed region, with every launch
     # bracketed by CUDA events on the (internal) stream it is launched on; the pipeline runs exactly as above
     # (seven kernels of neighbouring chunks overlap), so these are in-pipeline durations
@@ -823,6 +854,8 @@ def run_long(args):
     t_wall = time.perf_counter() - t_wall0
     clocks = sampler.stop() if rank == 0 else None
     launches = den.info["launches"] - launches0
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, call_frames, {"out": last_out[0] if c3 else out, "vad": vad})
     t = torch.tensor([total_ms], dtype=torch.float64, device=dev)
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)

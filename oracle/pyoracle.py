@@ -6,9 +6,12 @@ PARITY UNPINNED against nnnoiseless itself (see oracle/rnnoise_oracle.h).
 """
 from __future__ import annotations
 
+import atexit
 import ctypes as C
 import os
+import shutil
 import subprocess
+import tempfile
 
 import numpy as np
 
@@ -59,41 +62,23 @@ def build(force: bool = False) -> str:
     return _LIB_PATH
 
 
-_NATIVE_PATH = os.path.join(_HERE, "librnnoise_oracle_native.so")
+_native_path = None
 
 
-def _host_stamp() -> str:
-    """Identifies the machine and the source a native build belongs to: CPU model + ISA flags + source mtime."""
-    import hashlib
-    try:
-        with open("/proc/cpuinfo") as f:
-            cpu = "".join(l for l in f if l.startswith(("model name", "flags")) )[:20000]
-    except OSError:
-        cpu = "unknown"
-    src = os.path.join(_HERE, "rnnoise_oracle.c")
-    return hashlib.sha1((cpu + str(os.path.getmtime(src))).encode()).hexdigest()
-
-
-def build_native(force: bool = True) -> str:
-    """-O3 -march=native build of the same source for the CPU baseline.  Rebuilt on every machine that runs it (an
-    -march=native object must not travel between hosts: the stamp file names the CPU and the source it was built
-    from, and a library with another stamp -- e.g. one that came along in a gpurun snapshot -- is rebuilt)."""
-    src = os.path.join(_HERE, "rnnoise_oracle.c")
-    stamp_path = _NATIVE_PATH + ".stamp"
-    stamp = _host_stamp()
-    if not force and os.path.exists(_NATIVE_PATH) and os.path.exists(stamp_path):
-        try:
-            if open(stamp_path).read().strip() == stamp:
-                return _NATIVE_PATH
-        except OSError:
-            pass
-    tmp = _NATIVE_PATH + f".{os.getpid()}.tmp"
-    subprocess.check_call(["gcc", "-O3", "-march=native", "-fPIC", "-ffp-contract=off", "-fno-fast-math",
-                           "-std=c11", "-shared", "-o", tmp, src, "-lm", "-lpthread"])
-    os.replace(tmp, _NATIVE_PATH)
-    with open(stamp_path, "w") as f:
-        f.write(stamp)
-    return _NATIVE_PATH
+def build_native() -> str:
+    """-O3 -march=native build of the same source for the CPU baseline, compiled once per process into a private
+    temporary directory that is removed at exit: an -march=native object belongs to the CPU it was built on, and the
+    benchmark must run from a read-only tree."""
+    global _native_path
+    if _native_path is None:
+        d = tempfile.mkdtemp(prefix="crispy_oracle_native_")
+        atexit.register(shutil.rmtree, d, True)
+        path = os.path.join(d, "librnnoise_oracle_native.so")
+        subprocess.check_call(["gcc", "-O3", "-march=native", "-fPIC", "-ffp-contract=off", "-fno-fast-math",
+                               "-std=c11", "-shared", "-o", path, os.path.join(_HERE, "rnnoise_oracle.c"),
+                               "-lm", "-lpthread"])
+        _native_path = path
+    return _native_path
 
 
 _lib = None
@@ -104,8 +89,7 @@ def lib(native: bool = False) -> C.CDLL:
     global _lib
     if native:
         if "native" not in _libs:
-            build_native(force=False)
-            _libs["native"] = _declare(C.CDLL(_NATIVE_PATH))
+            _libs["native"] = _declare(C.CDLL(build_native()))
         return _libs["native"]
     if _lib is not None:
         return _lib
