@@ -56,6 +56,16 @@ extern "C" {
     fn crispy_ns_batch_state_size(b: *const CrispyNsBatch) -> usize;
     fn crispy_ns_batch_save_state(b: *mut CrispyNsBatch, buf: *mut c_void, len: usize) -> c_int;
     fn crispy_ns_batch_load_state(b: *mut CrispyNsBatch, buf: *const c_void, len: usize) -> c_int;
+    fn crispy_ns_process_streams_subset_host(
+        b: *mut CrispyNsBatch, streams: *const c_int, n_active: c_int, h_in: *const c_void, h_out: *mut c_void,
+        h_vad: *mut c_float, h_app: *const c_float, n_frames: c_int, in_stride: i64, out_stride: i64, vad_stride: i64,
+        app_stride: i64, flags: u32, volume: c_float,
+    ) -> c_int;
+    fn crispy_ns_batch_reset_streams(b: *mut CrispyNsBatch, streams: *const c_int, n: c_int, cuda_stream: *mut c_void) -> c_int;
+    fn crispy_ns_stream_state_size() -> usize;
+    fn crispy_ns_batch_save_streams(b: *mut CrispyNsBatch, streams: *const c_int, n: c_int, buf: *mut c_void, len: usize) -> c_int;
+    fn crispy_ns_batch_load_streams(b: *mut CrispyNsBatch, streams: *const c_int, n: c_int, buf: *const c_void, len: usize)
+                                    -> c_int;
     fn crispy_ns_batch_destroy(b: *mut CrispyNsBatch);
     fn crispy_ns_multi_create(model: *const CrispyNsModel, devices: *const c_int, n_devices: c_int, n_streams: c_int,
                               out: *mut *mut CrispyNsMulti) -> c_int;
@@ -204,6 +214,55 @@ impl BatchDenoiser {
     }
     pub fn load_state(&mut self, buf: &[u8]) -> Result<(), String> {
         let rc = unsafe { crispy_ns_batch_load_state(self.h, buf.as_ptr() as *const c_void, buf.len()) };
+        if rc != 0 {
+            return Err(last_error());
+        }
+        Ok(())
+    }
+    /// Streams that advance independently: row i of `input` / `output` (`n_frames * 480` unit-scale samples,
+    /// `stride` apart) is batch stream `streams[i]`; every other stream is left as it was.
+    pub fn process_streams_subset(&mut self, streams: &[i32], input: &[f32], output: &mut [f32], n_frames: usize,
+                                  stride: usize, volume: f32) -> Result<(), String> {
+        if let Some(rows) = streams.len().checked_sub(1) {
+            assert!(input.len() >= rows * stride + n_frames * FRAME_SIZE);
+            assert!(output.len() >= rows * stride + n_frames * FRAME_SIZE);
+        }
+        let rc = unsafe {
+            crispy_ns_process_streams_subset_host(self.h, streams.as_ptr(), streams.len() as c_int,
+                                                  input.as_ptr() as *const c_void, output.as_mut_ptr() as *mut c_void,
+                                                  std::ptr::null_mut(), std::ptr::null(), n_frames as c_int, stride as i64,
+                                                  stride as i64, 0, 0, CRISPY_NS_UNIT_SCALE, volume)
+        };
+        if rc != 0 {
+            return Err(last_error());
+        }
+        Ok(())
+    }
+    /// fresh DenoiseStates for the listed streams, ordered before the next call
+    pub fn reset_streams(&mut self, streams: &[i32]) -> Result<(), String> {
+        let rc = unsafe { crispy_ns_batch_reset_streams(self.h, streams.as_ptr(), streams.len() as c_int, std::ptr::null_mut()) };
+        if rc != 0 {
+            return Err(last_error());
+        }
+        Ok(())
+    }
+    /// one self-describing record per listed stream; it loads into any stream of any batch of this build
+    pub fn save_streams(&mut self, streams: &[i32]) -> Result<Vec<u8>, String> {
+        let n = streams.len() * unsafe { crispy_ns_stream_state_size() };
+        let mut buf = vec![0u8; n];
+        let rc = unsafe {
+            crispy_ns_batch_save_streams(self.h, streams.as_ptr(), streams.len() as c_int, buf.as_mut_ptr() as *mut c_void, n)
+        };
+        if rc != 0 {
+            return Err(last_error());
+        }
+        Ok(buf)
+    }
+    pub fn load_streams(&mut self, streams: &[i32], buf: &[u8]) -> Result<(), String> {
+        let rc = unsafe {
+            crispy_ns_batch_load_streams(self.h, streams.as_ptr(), streams.len() as c_int, buf.as_ptr() as *const c_void,
+                                         buf.len())
+        };
         if rc != 0 {
             return Err(last_error());
         }

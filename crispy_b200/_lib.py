@@ -33,6 +33,8 @@ SYMBOLS = [
     "crispy_ns_multi_create", "crispy_ns_multi_n_devices", "crispy_ns_multi_stream_range", "crispy_ns_multi_reset",
     "crispy_ns_multi_process_streams_host", "crispy_ns_multi_destroy", "crispy_ns_denoise_wav_files",
     "crispy_ns_measure_fp32",
+    "crispy_ns_process_streams_subset", "crispy_ns_process_streams_subset_host", "crispy_ns_batch_reset_streams",
+    "crispy_ns_stream_state_size", "crispy_ns_batch_save_streams", "crispy_ns_batch_load_streams",
 ]
 
 
@@ -79,6 +81,13 @@ def lib() -> C.CDLL:
     L.crispy_ns_batch_state_size.restype = C.c_size_t
     L.crispy_ns_batch_save_state.argtypes = [vp, vp, C.c_size_t]
     L.crispy_ns_batch_load_state.argtypes = [vp, vp, C.c_size_t]
+    ip = C.POINTER(C.c_int)
+    L.crispy_ns_process_streams_subset.argtypes = [vp, ip, C.c_int, vp, vp, vp, vp, C.c_int, i64, i64, i64, i64, u32, f32, vp]
+    L.crispy_ns_process_streams_subset_host.argtypes = [vp, ip, C.c_int, vp, vp, vp, vp, C.c_int, i64, i64, i64, i64, u32, f32]
+    L.crispy_ns_batch_reset_streams.argtypes = [vp, ip, C.c_int, vp]
+    L.crispy_ns_stream_state_size.restype = C.c_size_t
+    L.crispy_ns_batch_save_streams.argtypes = [vp, ip, C.c_int, vp, C.c_size_t]
+    L.crispy_ns_batch_load_streams.argtypes = [vp, ip, C.c_int, vp, C.c_size_t]
     L.crispy_ns_batch_info.argtypes = [vp, C.POINTER(C.c_int), C.POINTER(C.c_int), C.POINTER(i64), C.POINTER(i64)]
     L.crispy_ns_kernel_count.restype = C.c_int
     L.crispy_ns_kernel_name.argtypes = [C.c_int]

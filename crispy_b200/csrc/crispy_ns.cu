@@ -103,6 +103,39 @@ __global__ void __launch_bounds__(ns::kGroupThreads, NS_SYN_MINB) ns_synthesis_k
   ns::synthesis_body(p, *reinterpret_cast<ns::SpecSmem *>(smem_raw));
 }
 
+// Per-stream state rows by index (subset calls, per-stream reset, save / load of single streams): one CTA per row,
+// 16-byte accesses coalesced across the row's 11,136 bytes.  Row j of the launch moves src row (ids_on_src ? ids[j] :
+// first + j) to dst row (ids_on_src ? first + j : ids[j]); src == null writes zeros.  synthesis_mem (kStSynth) is
+// double buffered: dst's copy dst_cur receives src's copy src_cur, and dst's other copy src's other copy
+// (keep_stale) or zeros -- the other copy is scratch the next chunk writes before any read.
+constexpr int kRowIds = 960;  // ids per launch: the parameter block stays under 4 KB
+struct RowArgs {
+  float *dst;
+  const float *src;
+  int first, n, ids_on_src, src_cur, dst_cur, keep_stale;
+  int ids[kRowIds];
+};
+constexpr int kRowVec = ns::kStateFloats / 4;
+static_assert(ns::kStateFloats % 4 == 0 && ns::kStSynth % 4 == 0 && ns::kFrame % 4 == 0, "rows move as float4");
+__global__ void __launch_bounds__(256) ns_state_rows_kernel(const __grid_constant__ RowArgs a) {
+  const int j = blockIdx.x;
+  const long long s = a.ids_on_src ? a.ids[j] : a.first + j, d = a.ids_on_src ? a.first + j : a.ids[j];
+  const float4 *src = a.src ? reinterpret_cast<const float4 *>(a.src + s * ns::kStateFloats) : nullptr;
+  float4 *dst = reinterpret_cast<float4 *>(a.dst + d * ns::kStateFloats);
+  constexpr int syn0 = ns::kStSynth / 4, syn_len = ns::kFrame / 4;
+  for (int q = threadIdx.x; q < kRowVec; q += blockDim.x) {
+    int from = q;
+    bool zero = src == nullptr;
+    if (q >= syn0 && q < syn0 + 2 * syn_len) {
+      const int copy = (q - syn0) / syn_len, off = (q - syn0) % syn_len;
+      const int src_copy = copy == a.dst_cur ? a.src_cur : 1 - a.src_cur;
+      from = syn0 + src_copy * syn_len + off;
+      if (copy != a.dst_cur && !a.keep_stale) zero = true;
+    }
+    dst[q] = zero ? make_float4(0.f, 0.f, 0.f, 0.f) : src[from];
+  }
+}
+
 // a4/f2: out[s][n] = in[s][idx[n]-1] + (in[s][idx[n]] - in[s][idx[n]-1]) * frac[n], no FMA
 // contraction so the result is bit-identical to LinearResampler::process_sample (audio.rs:125-129).
 __global__ void __launch_bounds__(256) ns_linear_resample_kernel(const float *__restrict__ in, float *__restrict__ out,
@@ -436,6 +469,15 @@ struct crispy_ns_batch {
   cudaEvent_t e_start = nullptr;
   cudaEvent_t e_reset = nullptr;  // recorded by batch_reset_async; every internal stream waits for it once
   bool reset_pending = false;
+  // per-stream operations (subset calls, reset / save / load of listed streams).  d_rows: compact state rows, allocated
+  // at the first such operation.  Row copies run on the internal streams; e_rows marks the last one, and the next
+  // call's first kernel waits for it (rows_pending).  per_stream_ops: the streams no longer share one first frame, so
+  // a full call with CRISPY_NS_DROP_FIRST_FRAME is refused until the whole batch is reset or loaded.
+  float *d_rows = nullptr;
+  cudaEvent_t e_rows = nullptr;
+  bool rows_pending = false;
+  bool per_stream_ops = false;
+  int hp_exclusive_env = -1, hp_par_env = -1;  // $CRISPY_NS_HP_EXCLUSIVE / $CRISPY_NS_HP_PAR at batch_create, -1 unset
   cudaEvent_t e_k[kSlots][kNumKernels] = {};  // "kernel k of the chunk in this slot has finished"
   // optional per-kernel timing (crispy_ns_batch_profile): CUDA events around every launch, each on
   // the stream the kernel is launched on
@@ -517,6 +559,13 @@ static cudaError_t configure_kernels(int dev) {
   return e;
 }
 
+// K0's form for a call over n streams ($CRISPY_NS_HP_EXCLUSIVE / $CRISPY_NS_HP_PAR as read at batch_create win).  Both
+// forms give the same bits, so a subset call may pick the form for its own size.
+static void pick_hp_form(const crispy_ns_batch *b, int n, bool *exclusive, bool *par) {
+  *exclusive = b->hp_exclusive_env >= 0 ? b->hp_exclusive_env != 0 : n <= NS_HP_EXCLUSIVE_MAX_STREAMS;
+  *par = b->hp_par_env >= 0 ? b->hp_par_env != 0 : (NS_HP_PAR != 0 && *exclusive);
+}
+
 static cudaError_t prof_begin(crispy_ns_batch *b, int kernel, cudaStream_t s) {
   if (!b->prof_on) return cudaSuccess;
   crispy_ns_batch::ProfRec r;
@@ -550,16 +599,17 @@ struct RunHooks {
   cudaEvent_t all_done = nullptr;  // recorded after the call's last K5
 };
 
-// one kernel of the chunk described by p (n streams x nf frames) on stream sk
-static void launch_kernel(crispy_ns_batch *b, int k, ns::Params &p, int n, int nf, int groups, cudaStream_t sk) {
+// one kernel of the chunk described by p (n streams x nf frames) on stream sk; K0 in the form hp_par / hp_exclusive
+static void launch_kernel(crispy_ns_batch *b, int k, ns::Params &p, int n, int nf, int groups, cudaStream_t sk, bool hp_par,
+                          bool hp_exclusive) {
   switch (k) {
     case 0:
       // measurement aid only: skip the biquad once N chunks have run (the slots then still hold realistic signal)
       if (getenv("CRISPY_NS_EXPERIMENT_SKIP_HP") && b->chunks_done >= atoll(getenv("CRISPY_NS_EXPERIMENT_SKIP_HP"))) break;
-      if (b->hp_par)
-        ns_highpass_par_kernel<<<(n + 31) / 32, ns::kHpParThreads, b->hp_exclusive ? (size_t)kHpExclusiveSmem : sizeof(ns::HpParSmem), sk>>>(p);
+      if (hp_par)
+        ns_highpass_par_kernel<<<(n + 31) / 32, ns::kHpParThreads, hp_exclusive ? (size_t)kHpExclusiveSmem : sizeof(ns::HpParSmem), sk>>>(p);
       else
-        ns_highpass_kernel<<<(n + 31) / 32, ns::kHpThreads, b->hp_exclusive ? (size_t)kHpExclusiveSmem : sizeof(ns::HpSmem), sk>>>(p);
+        ns_highpass_kernel<<<(n + 31) / 32, ns::kHpThreads, hp_exclusive ? (size_t)kHpExclusiveSmem : sizeof(ns::HpSmem), sk>>>(p);
       break;
     case 1:
       ns_pitch_kernel<<<n * ((nf + kPitchRun - 1) / kPitchRun), kPitchThreads, sizeof(PitchShared), sk>>>(p);
@@ -602,12 +652,17 @@ static void launch_kernel(crispy_ns_batch *b, int k, ns::Params &p, int n, int n
 static int run_device(crispy_ns_batch *b, const void *d_in, void *d_out, float *d_vad, const float *d_app,
                       float *d_taps, int n_frames, int64_t in_stride, int64_t out_stride,
                       int64_t vad_stride, int64_t app_stride, uint32_t flags, float volume, cudaStream_t st,
-                      const RunHooks *hooks = nullptr) {
+                      const RunHooks *hooks = nullptr, int n_rows = 0) {
+  // n_rows > 0: a subset call over the first n_rows compact rows of d_rows (rows_gather put them there); it leaves
+  // frames_done alone
   if (!b || n_frames < 0) return fail(CRISPY_NS_EINVAL, "process_streams: bad argument");
   if (n_frames == 0) return CRISPY_NS_OK;  // an empty call touches nothing (its pointers may be null)
   if (!d_in || !d_out) return fail(CRISPY_NS_EINVAL, "process_streams: bad argument");
   if ((flags & CRISPY_NS_OUT_I16) && !(flags & CRISPY_NS_MIX_STEREO_I16) && volume != 1.0f)
     return fail(CRISPY_NS_EINVAL, "process_streams: CRISPY_NS_OUT_I16 is in 16-bit scale and takes no volume (use 1.0)");
+  if ((flags & CRISPY_NS_DROP_FIRST_FRAME) && b->per_stream_ops)
+    return fail(CRISPY_NS_EINVAL, "process_streams: CRISPY_NS_DROP_FIRST_FRAME after a per-stream operation: the streams no "
+                                  "longer share a first frame (reset or load the whole batch first)");
   NS_CUDA(cudaSetDevice(b->device));
   NS_CUDA(configure_kernels(b->device));
   ns::Params p;
@@ -617,7 +672,7 @@ static int run_device(crispy_ns_batch *b, const void *d_in, void *d_out, float *
   p.vad = d_vad;
   p.app = d_app;
   p.dbg = d_taps;
-  p.state = b->d_state;
+  p.state = n_rows > 0 ? b->d_rows : b->d_state;
   p.tables = b->d_tables;
   p.rnn_hdr = b->d_hdr;
   p.rnn_words = b->d_words;
@@ -627,17 +682,23 @@ static int run_device(crispy_ns_batch *b, const void *d_in, void *d_out, float *
   p.vad_stride = vad_stride;
   p.app_stride = app_stride;
   p.hp_stride = ns::kHist + (long long)b->chunk_cap * ns::kFrame;
-  p.n_streams = b->n_streams;
+  p.n_streams = n_rows > 0 ? n_rows : b->n_streams;
   p.n_frames_call = n_frames;
   p.chunk_cap = b->chunk_cap;
   p.out_frame_offset = ((flags & CRISPY_NS_DROP_FIRST_FRAME) && b->frames_done == 0) ? -1 : 0;
   p.flags = flags & 0xFFu;
   p.volume = volume;
-  const int n = b->n_streams;
+  const int n = p.n_streams;
   const int groups = (n + ns::kMmaStreams - 1) / ns::kMmaStreams;
+  bool hp_par = b->hp_par, hp_exclusive = b->hp_exclusive;
+  if (n_rows > 0) pick_hp_form(b, n, &hp_exclusive, &hp_par);
   if (b->reset_pending) {  // an asynchronous reset of the per-stream state is in flight on some caller stream
     for (int k = 0; k < kNumKernels; k++) NS_CUDA(cudaStreamWaitEvent(b->s_k[k], b->e_reset, 0));
     b->reset_pending = false;
+  }
+  if (b->rows_pending) {  // a per-stream row operation is in flight on the internal streams
+    NS_CUDA(cudaStreamWaitEvent(b->s_k[0], b->e_rows, 0));
+    b->rows_pending = false;
   }
   if (hooks) {
     NS_CUDA(cudaStreamWaitEvent(b->s_k[0], hooks->in_ready, 0));
@@ -667,7 +728,7 @@ static int run_device(crispy_ns_batch *b, const void *d_in, void *d_out, float *
       cudaStream_t sk = b->s_k[k];
       if (k > 0) NS_CUDA(cudaStreamWaitEvent(sk, b->e_k[slot][k - 1], 0));
       NS_CUDA(prof_begin(b, k, sk));
-      launch_kernel(b, k, p, n, nf, groups, sk);
+      launch_kernel(b, k, p, n, nf, groups, sk, hp_par, hp_exclusive);
       NS_CUDA(cudaGetLastError());
       NS_CUDA(prof_end(b, sk));
       NS_CUDA(cudaEventRecord(b->e_k[slot][k], sk));
@@ -682,7 +743,7 @@ static int run_device(crispy_ns_batch *b, const void *d_in, void *d_out, float *
   } else {
     NS_CUDA(cudaStreamWaitEvent(st, b->e_k[last_slot][kNumKernels - 1], 0));
   }
-  b->frames_done += n_frames;
+  if (n_rows == 0) b->frames_done += n_frames;
   return CRISPY_NS_OK;
 }
 
@@ -763,6 +824,8 @@ void batch_destroy(crispy_ns_batch *b) {
   cudaFree(b->d_words_tc5);
   cudaFree(b->d_bias_tc5);
   cudaFree(b->d_state);
+  cudaFree(b->d_rows);
+  if (b->e_rows) cudaEventDestroy(b->e_rows);
   for (int i = 0; i < kSlots; i++) {
     cudaFree(b->d_hp[i]);
     cudaFree(b->d_tab[i]);
@@ -854,9 +917,10 @@ int batch_create(const crispy_ns_model *model, int device, int n_streams, crispy
     // (profiles/r2_k4_tcgen05.md), so it stays opt-in (NS_RNN_TC5_MIN_STREAMS).
     // K0 alone on its SMs: $CRISPY_NS_HP_EXCLUSIVE = 1 / 0, default by batch size
     const char *hx = getenv("CRISPY_NS_HP_EXCLUSIVE");
-    b->hp_exclusive = hx ? atoi(hx) != 0 : n_streams <= NS_HP_EXCLUSIVE_MAX_STREAMS;
     const char *hpp = getenv("CRISPY_NS_HP_PAR");
-    b->hp_par = hpp ? atoi(hpp) != 0 : (NS_HP_PAR != 0 && b->hp_exclusive);
+    b->hp_exclusive_env = hx ? atoi(hx) != 0 : -1;
+    b->hp_par_env = hpp ? atoi(hpp) != 0 : -1;
+    pick_hp_form(b, n_streams, &b->hp_exclusive, &b->hp_par);
     const char *sel = getenv("CRISPY_NS_RNN");
     b->rnn_tc5 = sel ? (strcmp(sel, "tc5") == 0) : (n_streams >= NS_RNN_TC5_MIN_STREAMS);
     std::vector<uint8_t> w5;
@@ -908,6 +972,7 @@ int batch_reset(crispy_ns_batch *b) {
   NS_CUDA(cudaDeviceSynchronize());
   NS_CUDA(cudaMemset(b->d_state, 0, (size_t)b->n_streams * ns::kStateFloats * sizeof(float)));
   b->frames_done = 0;
+  b->per_stream_ops = false;
   return CRISPY_NS_OK;
 }
 int batch_reset_async(crispy_ns_batch *b, void *cuda_stream) {
@@ -917,6 +982,7 @@ int batch_reset_async(crispy_ns_batch *b, void *cuda_stream) {
   NS_CUDA(cudaEventRecord(b->e_reset, (cudaStream_t)cuda_stream));
   b->reset_pending = true;
   b->frames_done = 0;
+  b->per_stream_ops = false;
   return CRISPY_NS_OK;
 }
 int batch_n_streams(const crispy_ns_batch *b) { return b ? b->n_streams : 0; }
@@ -936,13 +1002,16 @@ int process_streams_debug(crispy_ns_batch *b, const void *d_in, void *d_out, flo
                     flags, volume, (cudaStream_t)cuda_stream);
 }
 
-int process_streams_host(crispy_ns_batch *b, const void *h_in, void *h_out, float *h_vad,
-                                   const float *h_app, int n_frames, int64_t in_stride,
-                                   int64_t out_stride, int64_t vad_stride, int64_t app_stride,
-                                   uint32_t flags, float volume) {
+// the host-pointer path over all streams, or (n_rows > 0) over the compact rows a subset call gathered
+static int run_host(crispy_ns_batch *b, const void *h_in, void *h_out, float *h_vad, const float *h_app, int n_frames,
+                    int64_t in_stride, int64_t out_stride, int64_t vad_stride, int64_t app_stride, uint32_t flags,
+                    float volume, int n_rows) {
   if (!b || n_frames < 0) return fail(CRISPY_NS_EINVAL, "process_streams_host: bad argument");
   if (n_frames == 0) return CRISPY_NS_OK;  // an empty call touches nothing (its pointers may be null)
   if (!h_in || !h_out) return fail(CRISPY_NS_EINVAL, "process_streams_host: bad argument");
+  if ((flags & CRISPY_NS_DROP_FIRST_FRAME) && b->per_stream_ops)
+    return fail(CRISPY_NS_EINVAL, "process_streams_host: CRISPY_NS_DROP_FIRST_FRAME after a per-stream operation: the "
+                                  "streams no longer share a first frame (reset or load the whole batch first)");
   NS_CUDA(cudaSetDevice(b->device));
   if (!b->s_in) {
     NS_CUDA(cudaStreamCreateWithFlags(&b->s_in, cudaStreamNonBlocking));
@@ -955,7 +1024,7 @@ int process_streams_host(crispy_ns_batch *b, const void *h_in, void *h_out, floa
     }
   }
   const size_t ie = in_elem(flags), oe = out_elem(flags);
-  const int n = b->n_streams;
+  const int n = n_rows > 0 ? n_rows : b->n_streams;
   // host chunk length in frames: a whole number of engine chunks, ~128 MiB of input per buffer
   long long ch = (128ll << 20) / ((long long)n * ns::kFrame * (long long)ie) / b->chunk_cap * b->chunk_cap;
   if (ch < b->chunk_cap) ch = b->chunk_cap;
@@ -1033,7 +1102,7 @@ int process_streams_host(crispy_ns_batch *b, const void *h_in, void *h_out, floa
     hooks.all_done = b->e_run[k];
     const int rc = run_device(b, b->d_in[k], b->d_out[k], h_vad ? b->d_vad[k] : nullptr,
                               use_app ? b->d_app[k] : nullptr, nullptr, (int)nf, row, row, nf, row, flags,
-                              volume, nullptr, &hooks);
+                              volume, nullptr, &hooks, n_rows);
     if (rc != CRISPY_NS_OK) return rc;
     NS_CUDA(cudaStreamWaitEvent(b->s_out, b->e_run[k], 0));
     if (nf_out > 0)
@@ -1048,6 +1117,13 @@ int process_streams_host(crispy_ns_batch *b, const void *h_in, void *h_out, floa
   NS_CUDA(cudaStreamSynchronize(b->s_out));
   NS_CUDA(cudaStreamSynchronize(b->s_in));
   return CRISPY_NS_OK;
+}
+
+int process_streams_host(crispy_ns_batch *b, const void *h_in, void *h_out, float *h_vad,
+                                   const float *h_app, int n_frames, int64_t in_stride,
+                                   int64_t out_stride, int64_t vad_stride, int64_t app_stride,
+                                   uint32_t flags, float volume) {
+  return run_host(b, h_in, h_out, h_vad, h_app, n_frames, in_stride, out_stride, vad_stride, app_stride, flags, volume, 0);
 }
 
 size_t batch_state_size(const crispy_ns_batch *b) {
@@ -1074,7 +1150,194 @@ int batch_load_state(crispy_ns_batch *b, const void *buf, size_t len) {
   NS_CUDA(cudaDeviceSynchronize());
   NS_CUDA(cudaMemcpy(b->d_state, (const char *)buf + 16, batch_state_size(b) - 16, cudaMemcpyHostToDevice));
   b->frames_done = hdr[1];
+  b->per_stream_ops = false;
   if ((b->chunks_done & 1) != sel) b->chunks_done += 1;  // synthesis_mem double buffer parity (ns_common.h kStSynth)
+  return CRISPY_NS_OK;
+}
+
+// ---- per-stream operations ---------------------------------------------------------------------------
+// Subset calls gather the listed state rows into d_rows, run the unchanged pipeline over them and scatter them back.
+// Ordering: every row copy sits on an internal stream behind the last K5 already enqueued (s_k[6] carries every K5, and
+// each chunk's K5 follows its K0 .. K4), and e_rows, recorded after it, is what the next call's K0 waits for.
+// synthesis_mem parity: every stream's current copy is copy (chunks_done & 1).  A subset call of k chunks leaves its
+// rows' current copy at (P + k) & 1; an odd k advances chunks_done once more (one workspace slot skipped, as
+// batch_load_state does) and the scatter puts that copy back at P, so the invariant holds for every stream.
+// A stream record is a 16-byte header and the state row with the current copy first and zeros in the other.
+static const char kStreamMagic[8] = {'C', 'R', 'N', 'S', 'S', 'T', 'R', '1'};
+constexpr size_t kStreamHeader = 16, kRowBytes = (size_t)ns::kStateFloats * sizeof(float);
+
+static int check_ids(const crispy_ns_batch *b, const int *ids, int n, const char *what) {
+  if (!b) return fail(CRISPY_NS_EINVAL, std::string(what) + ": null handle");
+  if (n < 0 || n > b->n_streams || (n > 0 && !ids))
+    return fail(CRISPY_NS_EINVAL, std::string(what) + ": the stream count must be in [0, n_streams] with a stream list");
+  std::vector<char> seen((size_t)b->n_streams, 0);
+  for (int i = 0; i < n; i++) {
+    if (ids[i] < 0 || ids[i] >= b->n_streams) return fail(CRISPY_NS_EINVAL, std::string(what) + ": stream id out of range");
+    if (seen[(size_t)ids[i]]) return fail(CRISPY_NS_EINVAL, std::string(what) + ": stream listed twice");
+    seen[(size_t)ids[i]] = 1;
+  }
+  return CRISPY_NS_OK;
+}
+
+// d_rows and e_rows exist, and the internal streams are ordered after an asynchronous whole-batch reset
+static int rows_prepare(crispy_ns_batch *b) {
+  NS_CUDA(cudaSetDevice(b->device));
+  if (!b->d_rows) NS_CUDA(cudaMalloc((void **)&b->d_rows, (size_t)b->n_streams * kRowBytes));
+  if (!b->e_rows) NS_CUDA(cudaEventCreateWithFlags(&b->e_rows, cudaEventDisableTiming));
+  if (b->reset_pending) {
+    for (int k = 0; k < kNumKernels; k++) NS_CUDA(cudaStreamWaitEvent(b->s_k[k], b->e_reset, 0));
+    b->reset_pending = false;
+  }
+  return CRISPY_NS_OK;
+}
+
+static int rows_launch(cudaStream_t s, float *dst, const float *src, const int *ids, int n,
+                       bool ids_on_src, int src_cur, int dst_cur, bool keep_stale) {
+  RowArgs a;
+  a.dst = dst;
+  a.src = src;
+  a.ids_on_src = ids_on_src;
+  a.src_cur = src_cur;
+  a.dst_cur = dst_cur;
+  a.keep_stale = keep_stale;
+  for (int first = 0; first < n; first += kRowIds) {
+    a.first = first;
+    a.n = n - first < kRowIds ? n - first : kRowIds;
+    memcpy(a.ids, ids + first, (size_t)a.n * sizeof(int));
+    ns_state_rows_kernel<<<a.n, 256, 0, s>>>(a);
+    NS_CUDA(cudaGetLastError());
+  }
+  return CRISPY_NS_OK;
+}
+
+// row operation on s_k[6] done: the next call waits for it
+static int rows_publish(crispy_ns_batch *b) {
+  NS_CUDA(cudaEventRecord(b->e_rows, b->s_k[kNumKernels - 1]));
+  b->rows_pending = true;
+  return CRISPY_NS_OK;
+}
+
+static int subset_check(crispy_ns_batch *b, const int *ids, int m, const void *in, const void *out, int n_frames,
+                        uint32_t flags, float volume, const char *what) {
+  if (int rc = check_ids(b, ids, m, what)) return rc;
+  if (n_frames < 0) return fail(CRISPY_NS_EINVAL, std::string(what) + ": bad argument");
+  if (flags & CRISPY_NS_DROP_FIRST_FRAME)
+    return fail(CRISPY_NS_EINVAL, std::string(what) + ": CRISPY_NS_DROP_FIRST_FRAME is not taken on subset calls");
+  if (m == 0 || n_frames == 0) return CRISPY_NS_OK;
+  if (!in || !out) return fail(CRISPY_NS_EINVAL, std::string(what) + ": bad argument");
+  if ((flags & CRISPY_NS_OUT_I16) && !(flags & CRISPY_NS_MIX_STEREO_I16) && volume != 1.0f)
+    return fail(CRISPY_NS_EINVAL, std::string(what) + ": CRISPY_NS_OUT_I16 is in 16-bit scale and takes no volume (use 1.0)");
+  return CRISPY_NS_OK;
+}
+
+// gather on s_k[0], behind everything enqueued so far (the previous call's scatter included)
+static int subset_begin(crispy_ns_batch *b, const int *ids, int m) {
+  if (int rc = rows_prepare(b)) return rc;
+  NS_CUDA(cudaEventRecord(b->e_rows, b->s_k[kNumKernels - 1]));
+  NS_CUDA(cudaStreamWaitEvent(b->s_k[0], b->e_rows, 0));
+  b->rows_pending = false;
+  return rows_launch(b->s_k[0], b->d_rows, b->d_state, ids, m, true, 0, 0, true);
+}
+
+// scatter on s_k[6] after the call's last K5, restoring the parity invariant
+static int subset_end(crispy_ns_batch *b, const int *ids, int m, int64_t chunks_before) {
+  const int64_t k = b->chunks_done - chunks_before;
+  if (k & 1) b->chunks_done += 1;
+  b->per_stream_ops = true;
+  if (int rc = rows_launch(b->s_k[kNumKernels - 1], b->d_state, b->d_rows, ids, m, false, (int)((chunks_before + k) & 1),
+                           (int)(chunks_before & 1), true))
+    return rc;
+  return rows_publish(b);
+}
+
+int process_streams_subset(crispy_ns_batch *b, const int *streams, int n_active, const void *d_in, void *d_out,
+                           float *d_vad, const float *d_app, int n_frames, int64_t in_stride, int64_t out_stride,
+                           int64_t vad_stride, int64_t app_stride, uint32_t flags, float volume, void *cuda_stream) {
+  if (int rc = subset_check(b, streams, n_active, d_in, d_out, n_frames, flags, volume, "process_streams_subset")) return rc;
+  if (n_active == 0 || n_frames == 0) return CRISPY_NS_OK;
+  const int64_t c0 = b->chunks_done;
+  if (int rc = subset_begin(b, streams, n_active)) return rc;
+  if (int rc = run_device(b, d_in, d_out, d_vad, d_app, nullptr, n_frames, in_stride, out_stride, vad_stride, app_stride,
+                          flags, volume, (cudaStream_t)cuda_stream, nullptr, n_active))
+    return rc;
+  if (int rc = subset_end(b, streams, n_active, c0)) return rc;
+  NS_CUDA(cudaStreamWaitEvent((cudaStream_t)cuda_stream, b->e_rows, 0));
+  return CRISPY_NS_OK;
+}
+
+int process_streams_subset_host(crispy_ns_batch *b, const int *streams, int n_active, const void *h_in, void *h_out,
+                                float *h_vad, const float *h_app, int n_frames, int64_t in_stride, int64_t out_stride,
+                                int64_t vad_stride, int64_t app_stride, uint32_t flags, float volume) {
+  if (int rc = subset_check(b, streams, n_active, h_in, h_out, n_frames, flags, volume, "process_streams_subset_host"))
+    return rc;
+  if (n_active == 0 || n_frames == 0) return CRISPY_NS_OK;
+  const int64_t c0 = b->chunks_done;
+  if (int rc = subset_begin(b, streams, n_active)) return rc;
+  if (int rc = run_host(b, h_in, h_out, h_vad, h_app, n_frames, in_stride, out_stride, vad_stride, app_stride, flags,
+                        volume, n_active))
+    return rc;
+  if (int rc = subset_end(b, streams, n_active, c0)) return rc;
+  NS_CUDA(cudaStreamSynchronize(b->s_k[kNumKernels - 1]));
+  return CRISPY_NS_OK;
+}
+
+int batch_reset_streams(crispy_ns_batch *b, const int *streams, int n, void *cuda_stream) {
+  if (int rc = check_ids(b, streams, n, "batch_reset_streams")) return rc;
+  if (n == 0) return CRISPY_NS_OK;
+  if (int rc = rows_prepare(b)) return rc;
+  cudaStream_t s6 = b->s_k[kNumKernels - 1];
+  NS_CUDA(cudaEventRecord(b->e_start, (cudaStream_t)cuda_stream));  // behind the caller's work, too
+  NS_CUDA(cudaStreamWaitEvent(s6, b->e_start, 0));
+  if (int rc = rows_launch(s6, b->d_state, nullptr, streams, n, false, 0, 0, false)) return rc;
+  b->per_stream_ops = true;
+  if (int rc = rows_publish(b)) return rc;
+  NS_CUDA(cudaStreamWaitEvent((cudaStream_t)cuda_stream, b->e_rows, 0));
+  return CRISPY_NS_OK;
+}
+
+size_t stream_state_size(void) { return kStreamHeader + kRowBytes; }
+
+int batch_save_streams(crispy_ns_batch *b, const int *streams, int n, void *buf, size_t len) {
+  if (int rc = check_ids(b, streams, n, "batch_save_streams")) return rc;
+  if ((n > 0 && !buf) || len < (size_t)n * stream_state_size())
+    return fail(CRISPY_NS_EINVAL, "batch_save_streams: the buffer must hold n * crispy_ns_stream_state_size() bytes");
+  if (n == 0) return CRISPY_NS_OK;
+  if (int rc = rows_prepare(b)) return rc;
+  cudaStream_t s6 = b->s_k[kNumKernels - 1];
+  if (int rc = rows_launch(s6, b->d_rows, b->d_state, streams, n, true, (int)(b->chunks_done & 1), 0, false)) return rc;
+  NS_CUDA(cudaMemcpy2DAsync((char *)buf + kStreamHeader, stream_state_size(), b->d_rows, kRowBytes, kRowBytes, (size_t)n,
+                            cudaMemcpyDeviceToHost, s6));
+  if (int rc = rows_publish(b)) return rc;
+  NS_CUDA(cudaStreamSynchronize(s6));
+  for (int i = 0; i < n; i++) {
+    uint8_t *h = (uint8_t *)buf + (size_t)i * stream_state_size();
+    const uint32_t words[2] = {(uint32_t)ns::kStateFloats, 0u};
+    memcpy(h, kStreamMagic, 8);
+    memcpy(h + 8, words, 8);
+  }
+  return CRISPY_NS_OK;
+}
+
+int batch_load_streams(crispy_ns_batch *b, const int *streams, int n, const void *buf, size_t len) {
+  if (int rc = check_ids(b, streams, n, "batch_load_streams")) return rc;
+  if ((n > 0 && !buf) || len != (size_t)n * stream_state_size())
+    return fail(CRISPY_NS_EINVAL, "batch_load_streams: the buffer must be n records of crispy_ns_stream_state_size() bytes");
+  for (int i = 0; i < n; i++) {
+    const uint8_t *h = (const uint8_t *)buf + (size_t)i * stream_state_size();
+    uint32_t words[2];
+    memcpy(words, h + 8, 8);
+    if (memcmp(h, kStreamMagic, 8) != 0 || words[0] != (uint32_t)ns::kStateFloats || words[1] != 0)
+      return fail(CRISPY_NS_EINVAL, "batch_load_streams: not a stream record of this build");
+  }
+  if (n == 0) return CRISPY_NS_OK;
+  if (int rc = rows_prepare(b)) return rc;
+  cudaStream_t s6 = b->s_k[kNumKernels - 1];
+  NS_CUDA(cudaMemcpy2DAsync(b->d_rows, kRowBytes, (const char *)buf + kStreamHeader, stream_state_size(), kRowBytes, (size_t)n,
+                            cudaMemcpyHostToDevice, s6));
+  if (int rc = rows_launch(s6, b->d_state, b->d_rows, streams, n, false, 0, (int)(b->chunks_done & 1), false)) return rc;
+  b->per_stream_ops = true;
+  if (int rc = rows_publish(b)) return rc;
+  NS_CUDA(cudaStreamSynchronize(s6));  // buf may be reused as soon as the call returns
   return CRISPY_NS_OK;
 }
 int batch_info(const crispy_ns_batch *b, int *streams_per_cta, int *n_ctas, int64_t *launches,
@@ -1190,7 +1453,7 @@ static int frame_graph(crispy_ns_state *st, int slot) {
   static_assert(kSlots % 2 == 0, "the synthesis_mem parity follows the slot");
   NS_CUDA(cudaStreamBeginCapture(st->s, cudaStreamCaptureModeThreadLocal));
   cudaMemcpyAsync(st->d_io, st->h_pin, ns::kFrame * sizeof(float), cudaMemcpyHostToDevice, st->s);
-  for (int k = 0; k < kNumKernels; k++) launch_kernel(b, k, p, 1, 1, 1, st->s);
+  for (int k = 0; k < kNumKernels; k++) launch_kernel(b, k, p, 1, 1, 1, st->s, b->hp_par, b->hp_exclusive);
   cudaMemcpyAsync(st->h_pin + 480, st->d_io + 480, 481 * sizeof(float), cudaMemcpyDeviceToHost, st->s);
   cudaGraph_t graph = nullptr;
   const cudaError_t e = cudaStreamEndCapture(st->s, &graph);

@@ -372,6 +372,111 @@ class BatchDenoiser:
                                                         vad.stride(0), app_stride, flags, volume))
         return out, vad
 
+    # ---- streams that advance independently (include/crispy_ns.h, per-stream section) -------------
+    def _ids(self, streams):
+        ids = np.ascontiguousarray(np.asarray(streams, dtype=np.int64).reshape(-1))
+        if ids.size and (ids.min() < 0 or ids.max() >= self.n_streams):
+            raise CrispyNsError("stream id out of range")
+        ids = ids.astype(np.int32)
+        return ids, ids.ctypes.data_as(C.POINTER(C.c_int))
+
+    def _subset_io(self, n_rows, n_frames, in_dtype, unit_scale, drop_first_frame, out, vad, out_i16, mix_stereo_i16,
+                   device):
+        import torch
+        flags = (IN_I16 if in_dtype == torch.int16 else 0) | (UNIT_SCALE if unit_scale else 0)
+        if drop_first_frame:
+            flags |= DROP_FIRST_FRAME  # refused by the library: the caller drops a stream's first frame itself
+        n_samples = n_frames * FRAME_SIZE
+        if mix_stereo_i16:
+            flags |= MIX_STEREO_I16
+            if out is None:
+                out = torch.zeros((n_rows, n_samples, 2), dtype=torch.int16, device=device)
+            out_stride = out.stride(0) // 2
+        else:
+            if out_i16:
+                flags |= OUT_I16
+            if out is None:
+                out = torch.zeros((n_rows, n_samples), dtype=torch.int16 if out_i16 else torch.float32, device=device)
+            out_stride = out.stride(0)
+        if vad is None:
+            vad = torch.zeros((n_rows, n_frames), dtype=torch.float32, device=device)
+        return flags, out, out_stride, vad
+
+    def process_streams_subset(self, streams, x, *, unit_scale: bool = True, volume: float = 1.0,
+                               drop_first_frame: bool = False, out=None, vad=None, out_i16: bool = False,
+                               app=None, mix_stereo_i16: bool = False, input_rate: float = SAMPLE_RATE,
+                               front_end: str = "linear"):
+        """As process_streams for the listed streams only: row i of x (CUDA tensor [len(streams), n_frames*480]) is
+        stream streams[i]; every other stream's state stays as it was.  Asynchronous on the current torch stream.
+        drop_first_frame is refused (the caller drops a stream's first frame)."""
+        import torch
+        if abs(float(input_rate) - SAMPLE_RATE) >= 1.0:
+            if front_end not in ("linear", "sinc"):
+                raise CrispyNsError("front_end must be 'linear' or 'sinc'")
+            x = (sinc_resample(x, int(round(input_rate)), int(SAMPLE_RATE)) if front_end == "sinc"
+                 else linear_resample(x, float(input_rate), float(SAMPLE_RATE)))
+        ids, ptr = self._ids(streams)
+        if not x.is_cuda or x.dim() != 2 or x.stride(1) != 1 or x.shape[0] != ids.size:
+            raise CrispyNsError("process_streams_subset needs a CUDA [len(streams), n_samples] tensor")
+        if x.dtype not in (torch.float32, torch.int16):
+            raise CrispyNsError("process_streams_subset input must be float32 or int16")
+        n_frames = x.shape[1] // FRAME_SIZE
+        flags, out, out_stride, vad = self._subset_io(ids.size, n_frames, x.dtype, unit_scale, drop_first_frame, out,
+                                                      vad, out_i16, mix_stereo_i16, x.device)
+        app_ptr, app_stride = None, 0
+        if app is not None:
+            if not app.is_cuda or app.dtype != torch.float32 or app.stride(1) != 1:
+                raise CrispyNsError("app audio must be a CUDA float32 tensor")
+            app_ptr, app_stride = app.data_ptr(), app.stride(0)
+        st = torch.cuda.current_stream(x.device).cuda_stream
+        check(_lib.lib().crispy_ns_process_streams_subset(self._h, ptr, int(ids.size), x.data_ptr(), out.data_ptr(),
+                                                          vad.data_ptr(), app_ptr, n_frames, x.stride(0), out_stride,
+                                                          vad.stride(0), app_stride, flags, volume, st))
+        return out, vad
+
+    def process_streams_subset_host(self, streams, x, *, unit_scale: bool = True, volume: float = 1.0,
+                                    drop_first_frame: bool = False, out=None, vad=None, out_i16: bool = False,
+                                    app=None, mix_stereo_i16: bool = False):
+        """As process_streams_host for the listed streams only (row i of the host tensor x is stream streams[i])."""
+        import torch
+        ids, ptr = self._ids(streams)
+        xt = torch.as_tensor(x)
+        if xt.is_cuda or xt.dim() != 2 or xt.stride(1) != 1 or xt.shape[0] != ids.size:
+            raise CrispyNsError("process_streams_subset_host needs a host [len(streams), n_samples] tensor")
+        if xt.dtype not in (torch.float32, torch.int16):
+            raise CrispyNsError("process_streams_subset_host input must be float32 or int16")
+        n_frames = xt.shape[1] // FRAME_SIZE
+        flags, out, out_stride, vad = self._subset_io(ids.size, n_frames, xt.dtype, unit_scale, drop_first_frame, out,
+                                                      vad, out_i16, mix_stereo_i16, "cpu")
+        app_ptr, app_stride = None, 0
+        if app is not None:
+            app = torch.as_tensor(app)
+            app_ptr, app_stride = app.data_ptr(), app.stride(0)
+        check(_lib.lib().crispy_ns_process_streams_subset_host(self._h, ptr, int(ids.size), xt.data_ptr(), out.data_ptr(),
+                                                               vad.data_ptr(), app_ptr, n_frames, xt.stride(0),
+                                                               out_stride, vad.stride(0), app_stride, flags, volume))
+        return out, vad
+
+    def reset_streams(self, streams) -> None:
+        """Fresh DenoiseStates for the listed streams, on the current torch CUDA stream (no host sync)."""
+        import torch
+        ids, ptr = self._ids(streams)
+        st = torch.cuda.current_stream(self.device).cuda_stream
+        check(_lib.lib().crispy_ns_batch_reset_streams(self._h, ptr, int(ids.size), st))
+
+    def save_streams(self, streams) -> bytes:
+        """One self-describing record per listed stream (stream_state_size() bytes each), concatenated."""
+        ids, ptr = self._ids(streams)
+        n = int(ids.size) * stream_state_size()
+        buf = C.create_string_buffer(max(n, 1))
+        check(_lib.lib().crispy_ns_batch_save_streams(self._h, ptr, int(ids.size), buf, n))
+        return buf.raw[:n]
+
+    def load_streams(self, streams, blob: bytes) -> None:
+        """Put the records of save_streams (from any batch of this build) into the listed streams."""
+        ids, ptr = self._ids(streams)
+        check(_lib.lib().crispy_ns_batch_load_streams(self._h, ptr, int(ids.size), blob, len(blob)))
+
     # ---- bookkeeping ----------------------------------------------------------------------------
     @property
     def info(self) -> dict:
@@ -420,6 +525,11 @@ class BatchDenoiser:
                 _lib.lib().crispy_ns_batch_destroy(self._h)
         except Exception:
             pass
+
+
+def stream_state_size() -> int:
+    """Bytes of one stream record of BatchDenoiser.save_streams."""
+    return int(_lib.lib().crispy_ns_stream_state_size())
 
 
 class MultiDenoiser:

@@ -121,6 +121,44 @@ int crispy_ns_debug_floats(void);
 size_t crispy_ns_batch_state_size(const crispy_ns_batch *b);
 int crispy_ns_batch_save_state(crispy_ns_batch *b, void *buf, size_t len);
 int crispy_ns_batch_load_state(crispy_ns_batch *b, const void *buf, size_t len);
+
+/* ---- streams that advance independently: calls over a subset of the batch, and reset / checkpoint / resume of
+ * single streams (recordings of different lengths sharing slots, live streams that have a frame now, a recording
+ * moved to another batch or GPU).  A stream's results do not depend on which other streams share a call.
+ *   - streams[i] (host array, distinct ids, each in [0, n_streams)) is the batch stream whose samples are row i of
+ *     d_in / d_out / d_vad / d_app; every other stream's DenoiseState is left bit for bit as it was.  The array may
+ *     be reused as soon as the call returns.
+ *   - Geometry, flags and volume as crispy_ns_process_streams / _host, except that CRISPY_NS_DROP_FIRST_FRAME is
+ *     refused (the caller drops a stream's first frame itself).
+ *   - Arguments are checked before anything is enqueued: a null handle, n_active outside [0, n_streams], an id out of
+ *     range or listed twice, CRISPY_NS_DROP_FIRST_FRAME, or a record of the wrong length or magic give
+ *     CRISPY_NS_EINVAL and change no state.  n_active == 0 or n_frames == 0 touches nothing.
+ *   - frames_done (crispy_ns_batch_info) counts full-batch frames only: subset calls and per-stream resets and loads
+ *     leave it alone.  After any of them a full-batch call with CRISPY_NS_DROP_FIRST_FRAME is refused
+ *     (CRISPY_NS_EINVAL) until the next crispy_ns_batch_reset, _reset_async or _load_state.
+ *   - Ordering: the state rows are copied on the batch's own streams, after every call already enqueued and before
+ *     the next one, whichever CUDA stream that call is made on.  The device call is asynchronous on cuda_stream,
+ *     which waits for the call's last kernel; a subset call ends with its pipeline drained.
+ * ---- */
+int crispy_ns_process_streams_subset(crispy_ns_batch *b, const int *streams, int n_active, const void *d_in,
+                                     void *d_out, float *d_vad, const float *d_app, int n_frames,
+                                     int64_t in_stride, int64_t out_stride, int64_t vad_stride,
+                                     int64_t app_stride, uint32_t flags, float volume, void *cuda_stream);
+/* host pointers, synchronous, copies pipelined as in crispy_ns_process_streams_host */
+int crispy_ns_process_streams_subset_host(crispy_ns_batch *b, const int *streams, int n_active, const void *h_in,
+                                          void *h_out, float *h_vad, const float *h_app, int n_frames,
+                                          int64_t in_stride, int64_t out_stride, int64_t vad_stride,
+                                          int64_t app_stride, uint32_t flags, float volume);
+/* fresh DenoiseState for the listed streams only; asynchronous: ordered after the work already on cuda_stream and
+ * every call already enqueued, and before the batch's next call; cuda_stream waits for it */
+int crispy_ns_batch_reset_streams(crispy_ns_batch *b, const int *streams, int n, void *cuda_stream);
+/* one self-describing record per listed stream (host buffers, synchronous): a 16-byte header ("CRNSSTR1", the state's
+ * float count, 0) and the stream's DenoiseState -- 11,152 bytes in this build.  A record loads into any stream of
+ * any batch of this build; save_streams needs len >= n records, load_streams exactly n records. */
+size_t crispy_ns_stream_state_size(void);
+int crispy_ns_batch_save_streams(crispy_ns_batch *b, const int *streams, int n, void *buf, size_t len);
+int crispy_ns_batch_load_streams(crispy_ns_batch *b, const int *streams, int n, const void *buf, size_t len);
+
 /* launch geometry + bookkeeping: streams per recurrent-core CTA, frames per engine chunk
  * ($CRISPY_NS_CHUNK_FRAMES overrides the default at batch_create), kernels launched so far,
  * frames processed per stream */

@@ -333,6 +333,28 @@ class BatchDenoiser {
   }
   void load_state(const std::vector<std::uint8_t> &b) { detail::check(crispy_ns_batch_load_state(h_, b.data(), b.size())); }
   void reset() { detail::check(crispy_ns_batch_reset(h_)); }
+
+  // Streams that advance independently: row i of input / output / vad (n_frames per row) is batch stream streams[i];
+  // every other stream is left as it was.  Unit-scale f32, host pointers, synchronous.
+  void process_streams_subset(const std::vector<int> &streams, const float *input, float *output, float *vad,
+                              int n_frames, std::int64_t stride, float volume = 1.0f) {
+    detail::check(crispy_ns_process_streams_subset_host(h_, streams.data(), (int)streams.size(), input, output, vad,
+                                                        nullptr, n_frames, stride, stride, vad ? n_frames : 0, 0,
+                                                        CRISPY_NS_UNIT_SCALE, volume));
+  }
+  // fresh DenoiseStates for the listed streams (ordered before the next call; cuda_stream waits for it)
+  void reset_streams(const std::vector<int> &streams, void *cuda_stream = nullptr) {
+    detail::check(crispy_ns_batch_reset_streams(h_, streams.data(), (int)streams.size(), cuda_stream));
+  }
+  // one record of crispy_ns_stream_state_size() bytes per listed stream; loads into any stream of any batch
+  std::vector<std::uint8_t> save_streams(const std::vector<int> &streams) {
+    std::vector<std::uint8_t> b(streams.size() * crispy_ns_stream_state_size());
+    detail::check(crispy_ns_batch_save_streams(h_, streams.data(), (int)streams.size(), b.data(), b.size()));
+    return b;
+  }
+  void load_streams(const std::vector<int> &streams, const std::vector<std::uint8_t> &b) {
+    detail::check(crispy_ns_batch_load_streams(h_, streams.data(), (int)streams.size(), b.data(), b.size()));
+  }
   crispy_ns_batch *get() { return h_; }
 
  private:
