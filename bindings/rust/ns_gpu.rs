@@ -41,9 +41,19 @@ pub const CRISPY_NS_UNIT_SCALE: u32 = 1 << 2;
 pub const CRISPY_NS_MIX_STEREO_I16: u32 = 1 << 3;
 pub const CRISPY_NS_DROP_FIRST_FRAME: u32 = 1 << 8;
 
+/// numerics of a model (crispy_ns_model_set_numerics): the sum order of the pitch path's inner products | the biquad's
+/// arithmetic.  0 is xiph's C; every handle created from the model copies the setting.
+pub const CRISPY_NS_SUM_SEQUENTIAL: u32 = 0;
+pub const CRISPY_NS_SUM_DOT4: u32 = 1;
+pub const CRISPY_NS_SUM_DOT4_XCORR: u32 = 2;
+pub const CRISPY_NS_SUM_MASK: u32 = 3;
+pub const CRISPY_NS_BIQUAD_F32: u32 = 1 << 4;
+
 extern "C" {
     fn crispy_ns_last_error() -> *const c_char;
     fn crispy_ns_device_count() -> c_int;
+    pub fn crispy_ns_model_set_numerics(m: *mut CrispyNsModel, numerics: u32) -> c_int;
+    pub fn crispy_ns_model_numerics(m: *const CrispyNsModel) -> u32;
     fn crispy_ns_create(model: *const CrispyNsModel, device: c_int, out: *mut *mut CrispyNsState) -> c_int;
     fn crispy_ns_process_frame(st: *mut CrispyNsState, out480: *mut c_float, in480: *const c_float, vad: *mut c_float) -> c_int;
     fn crispy_ns_reset(st: *mut CrispyNsState) -> c_int;

@@ -16,6 +16,13 @@ UNIT_SCALE = 1 << 2
 MIX_STEREO_I16 = 1 << 3
 DROP_FIRST_FRAME = 1 << 8
 
+# numerics of a model (crispy_ns_model_set_numerics): sum order of the pitch path's inner products | biquad arithmetic
+SUM_SEQUENTIAL = 0
+SUM_DOT4 = 1
+SUM_DOT4_XCORR = 2
+SUM_MASK = 3
+BIQUAD_F32 = 1 << 4
+
 # every symbol include/crispy_ns.h declares
 SYMBOLS = [
     "crispy_ns_frame_size", "crispy_ns_last_error", "crispy_ns_device_count",
@@ -35,6 +42,7 @@ SYMBOLS = [
     "crispy_ns_measure_fp32",
     "crispy_ns_process_streams_subset", "crispy_ns_process_streams_subset_host", "crispy_ns_batch_reset_streams",
     "crispy_ns_stream_state_size", "crispy_ns_batch_save_streams", "crispy_ns_batch_load_streams",
+    "crispy_ns_model_set_numerics", "crispy_ns_model_numerics",
 ]
 
 
@@ -64,6 +72,9 @@ def lib() -> C.CDLL:
     L.crispy_ns_model_to_bytes.argtypes = [vp, C.c_char_p, C.c_size_t, C.POINTER(C.c_size_t)]
     L.crispy_ns_model_destroy.argtypes = [vp]
     L.crispy_ns_model_destroy.restype = None
+    L.crispy_ns_model_set_numerics.argtypes = [vp, u32]
+    L.crispy_ns_model_numerics.argtypes = [vp]
+    L.crispy_ns_model_numerics.restype = u32
     L.crispy_ns_create.argtypes = [vp, C.c_int, vpp]
     L.crispy_ns_process_frame.argtypes = [vp, vp, vp, C.POINTER(f32)]
     L.crispy_ns_reset.argtypes = [vp]

@@ -56,21 +56,45 @@ constexpr int kScanWarps = 4;
 // The second is the faster kernel (isolated 613 -> 424 us per 32,768 frames) and wins wherever K0 bounds the pipeline
 // (small batches, where it also has its SMs to itself); beside the pitch CTAs of a full batch its eight warps cost the
 // parallel kernels what its shorter run gives back, so the first form stays there (crispy_ns_batch::hp_par).
+// F32: the biquad in f32 arithmetic alone (CRISPY_NS_BIQUAD_F32); the parallel form speculates the f64 expression only
+template <bool F32>
 __global__ void __launch_bounds__(ns::kHpThreads) ns_highpass_kernel(const __grid_constant__ ns::Params p) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
-  ns::highpass_body(p, *reinterpret_cast<ns::HpSmem *>(smem_raw));
+  ns::highpass_body<F32>(p, *reinterpret_cast<ns::HpSmem *>(smem_raw));
 }
 __global__ void __launch_bounds__(ns::kHpParThreads) ns_highpass_par_kernel(const __grid_constant__ ns::Params p) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   ns::highpass_par_body(p, *reinterpret_cast<ns::HpParSmem *>(smem_raw));
 }
+// SP: the summation policy of the pitch path's inner products (CRISPY_NS_SUM_*; the second generation knows only 0)
+template <int SP>
 __global__ void __launch_bounds__(kPitchThreads) ns_pitch_kernel(const __grid_constant__ ns::Params p) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
 #ifndef NS_PITCH_V7
-  ns::pitch_body<kPitchRun, kPitchThreads>(p, *reinterpret_cast<PitchShared *>(smem_raw));
+  ns::pitch_body<kPitchRun, kPitchThreads, SP>(p, *reinterpret_cast<PitchShared *>(smem_raw));
 #else
+  static_assert(SP == 0, "ns_pitch7.cuh sums in the sequential order only");
   ns::pitch_body7<kPitchRun, kPitchThreads>(p, *reinterpret_cast<PitchShared *>(smem_raw));
 #endif
+}
+#ifndef NS_PITCH_V7
+constexpr int kPitchPolicies = 3;
+#else
+constexpr int kPitchPolicies = 1;
+#endif
+typedef void (*KernelFn)(ns::Params);
+static KernelFn pitch_kernel(uint32_t numerics) {
+#ifndef NS_PITCH_V7
+  switch (numerics & CRISPY_NS_SUM_MASK) {
+    case CRISPY_NS_SUM_DOT4: return ns_pitch_kernel<1>;
+    case CRISPY_NS_SUM_DOT4_XCORR: return ns_pitch_kernel<2>;
+    default: break;
+  }
+#endif
+  return ns_pitch_kernel<0>;
+}
+static KernelFn highpass_kernel(uint32_t numerics) {
+  return (numerics & CRISPY_NS_BIQUAD_F32) ? ns_highpass_kernel<true> : ns_highpass_kernel<false>;
 }
 __global__ void __launch_bounds__(32 * kScanWarps) ns_pitchscan_kernel(const __grid_constant__ ns::Params p) {
   ns::pitchscan_body(p, kScanWarps);
@@ -433,6 +457,7 @@ static int guard(const char *what, F &&body) noexcept {
 
 struct crispy_ns_model {
   ns::Model m;
+  uint32_t numerics = 0;  // crispy_ns_model_set_numerics; not part of the blob
 };
 
 constexpr int kSlots = 8;    // workspace slots: chunk c uses slot c % kSlots
@@ -456,6 +481,7 @@ struct crispy_ns_batch {
   uint8_t *d_words_tc5 = nullptr;
   float *d_bias_tc5 = nullptr;
   bool rnn_tc5 = false;
+  uint32_t numerics = 0;      // the model's crispy_ns_model_set_numerics at batch_create: K0's biquad form, K1's sum order
   bool hp_exclusive = false;  // K0 alone on its SMs (kHpExclusiveSmem)
   bool hp_par = false;        // K0 parallel in time (ns_highpass_par_kernel); $CRISPY_NS_HP_PAR overrides
   float *d_state = nullptr;
@@ -542,11 +568,13 @@ static cudaError_t configure_kernels(int dev) {
   static std::map<int, bool> configured;
   std::lock_guard<std::mutex> lk(mu);
   if (configured[dev]) return cudaSuccess;
-  cudaError_t e = cudaFuncSetAttribute(ns_highpass_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kHpExclusiveSmem);
+  cudaError_t e = cudaFuncSetAttribute(ns_highpass_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kHpExclusiveSmem);
+  if (e == cudaSuccess)
+    e = cudaFuncSetAttribute(ns_highpass_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kHpExclusiveSmem);
   if (e == cudaSuccess)
     e = cudaFuncSetAttribute(ns_highpass_par_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kHpExclusiveSmem);
-  if (e == cudaSuccess) e = cudaFuncSetAttribute(ns_pitch_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                       (int)sizeof(PitchShared));
+  for (int sp = 0; sp < kPitchPolicies && e == cudaSuccess; sp++)
+    e = cudaFuncSetAttribute(pitch_kernel((uint32_t)sp), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(PitchShared));
   if (e == cudaSuccess)
     e = cudaFuncSetAttribute(ns_spectrum_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(ns::SpecSmem));
   if (e == cudaSuccess)
@@ -560,10 +588,13 @@ static cudaError_t configure_kernels(int dev) {
 }
 
 // K0's form for a call over n streams ($CRISPY_NS_HP_EXCLUSIVE / $CRISPY_NS_HP_PAR as read at batch_create win).  Both
-// forms give the same bits, so a subset call may pick the form for its own size.
+// forms give the same bits, so a subset call may pick the form for its own size.  The parallel form speculates the f64
+// expression only: under CRISPY_NS_BIQUAD_F32 the single recursion warp runs (its f32 chain is a few dependent f32
+// operations a sample instead of the f64 chain's 74 cycles).
 static void pick_hp_form(const crispy_ns_batch *b, int n, bool *exclusive, bool *par) {
   *exclusive = b->hp_exclusive_env >= 0 ? b->hp_exclusive_env != 0 : n <= NS_HP_EXCLUSIVE_MAX_STREAMS;
   *par = b->hp_par_env >= 0 ? b->hp_par_env != 0 : (NS_HP_PAR != 0 && *exclusive);
+  if (b->numerics & CRISPY_NS_BIQUAD_F32) *par = false;
 }
 
 static cudaError_t prof_begin(crispy_ns_batch *b, int kernel, cudaStream_t s) {
@@ -609,10 +640,10 @@ static void launch_kernel(crispy_ns_batch *b, int k, ns::Params &p, int n, int n
       if (hp_par)
         ns_highpass_par_kernel<<<(n + 31) / 32, ns::kHpParThreads, hp_exclusive ? (size_t)kHpExclusiveSmem : sizeof(ns::HpParSmem), sk>>>(p);
       else
-        ns_highpass_kernel<<<(n + 31) / 32, ns::kHpThreads, hp_exclusive ? (size_t)kHpExclusiveSmem : sizeof(ns::HpSmem), sk>>>(p);
+        highpass_kernel(b->numerics)<<<(n + 31) / 32, ns::kHpThreads, hp_exclusive ? (size_t)kHpExclusiveSmem : sizeof(ns::HpSmem), sk>>>(p);
       break;
     case 1:
-      ns_pitch_kernel<<<n * ((nf + kPitchRun - 1) / kPitchRun), kPitchThreads, sizeof(PitchShared), sk>>>(p);
+      pitch_kernel(b->numerics)<<<n * ((nf + kPitchRun - 1) / kPitchRun), kPitchThreads, sizeof(PitchShared), sk>>>(p);
       break;
     case 2:
       ns_pitchscan_kernel<<<(n + kScanWarps - 1) / kScanWarps, 32 * kScanWarps, 0, sk>>>(p);
@@ -794,6 +825,14 @@ int model_to_bytes(const crispy_ns_model *m, void *buf, size_t cap, size_t *need
   return CRISPY_NS_OK;
 }
 void model_destroy(crispy_ns_model *m) { delete m; }
+int model_set_numerics(crispy_ns_model *m, uint32_t numerics) {
+  if (!m) return fail(CRISPY_NS_EINVAL, "model_set_numerics: model is null");
+  if ((numerics & ~(uint32_t)(CRISPY_NS_SUM_MASK | CRISPY_NS_BIQUAD_F32)) || (numerics & CRISPY_NS_SUM_MASK) == CRISPY_NS_SUM_MASK)
+    return fail(CRISPY_NS_EINVAL, "model_set_numerics: unknown bits, or sum order 3");
+  m->numerics = numerics;
+  return CRISPY_NS_OK;
+}
+uint32_t model_numerics(const crispy_ns_model *m) { return m ? m->numerics : 0u; }
 
 static int default_model(ns::Model &m) {
   const char *path = getenv("CRISPY_NS_WEIGHTS");
@@ -859,6 +898,11 @@ int batch_create(const crispy_ns_model *model, int device, int n_streams, crispy
   const int ndev = device_count();
   if (ndev == 0) return fail(CRISPY_NS_ENODEV, "no CUDA device: libcrispy_ns has no CPU fallback");
   if (device < 0 || device >= ndev) return fail(CRISPY_NS_ENODEV, "device index out of range");
+  const uint32_t numerics = model_numerics(model);
+#ifdef NS_PITCH_V7
+  if (numerics & CRISPY_NS_SUM_MASK)
+    return fail(CRISPY_NS_EINVAL, "batch_create: this build's pitch kernel (NS_PITCH_V7) sums in the sequential order only");
+#endif
   ns::Model local;
   const ns::Model *m = nullptr;
   if (model) {
@@ -875,6 +919,7 @@ int batch_create(const crispy_ns_model *model, int device, int n_streams, crispy
   if (!b) return fail(CRISPY_NS_ENOMEM, "out of memory");
   b->device = device;
   b->n_streams = n_streams;
+  b->numerics = numerics;
   b->n_sms = prop.multiProcessorCount;
   b->chunk_cap = default_chunk_cap(n_streams);
   if (const char *e = getenv("CRISPY_NS_SYN_RUN")) b->syn_run_override = atoi(e);
@@ -1162,7 +1207,8 @@ int batch_load_state(crispy_ns_batch *b, const void *buf, size_t len) {
 // synthesis_mem parity: every stream's current copy is copy (chunks_done & 1).  A subset call of k chunks leaves its
 // rows' current copy at (P + k) & 1; an odd k advances chunks_done once more (one workspace slot skipped, as
 // batch_load_state does) and the scatter puts that copy back at P, so the invariant holds for every stream.
-// A stream record is a 16-byte header and the state row with the current copy first and zeros in the other.
+// A stream record is a 16-byte header and the state row with the current copy first and zeros in the other.  The
+// header's last word is the batch's numerics: a state evolved under one arithmetic does not continue under another.
 static const char kStreamMagic[8] = {'C', 'R', 'N', 'S', 'S', 'T', 'R', '1'};
 constexpr size_t kStreamHeader = 16, kRowBytes = (size_t)ns::kStateFloats * sizeof(float);
 
@@ -1311,7 +1357,7 @@ int batch_save_streams(crispy_ns_batch *b, const int *streams, int n, void *buf,
   NS_CUDA(cudaStreamSynchronize(s6));
   for (int i = 0; i < n; i++) {
     uint8_t *h = (uint8_t *)buf + (size_t)i * stream_state_size();
-    const uint32_t words[2] = {(uint32_t)ns::kStateFloats, 0u};
+    const uint32_t words[2] = {(uint32_t)ns::kStateFloats, b->numerics};
     memcpy(h, kStreamMagic, 8);
     memcpy(h + 8, words, 8);
   }
@@ -1326,8 +1372,10 @@ int batch_load_streams(crispy_ns_batch *b, const int *streams, int n, const void
     const uint8_t *h = (const uint8_t *)buf + (size_t)i * stream_state_size();
     uint32_t words[2];
     memcpy(words, h + 8, 8);
-    if (memcmp(h, kStreamMagic, 8) != 0 || words[0] != (uint32_t)ns::kStateFloats || words[1] != 0)
+    if (memcmp(h, kStreamMagic, 8) != 0 || words[0] != (uint32_t)ns::kStateFloats)
       return fail(CRISPY_NS_EINVAL, "batch_load_streams: not a stream record of this build");
+    if (words[1] != b->numerics)
+      return fail(CRISPY_NS_EINVAL, "batch_load_streams: the record was saved under other numerics than the batch's");
   }
   if (n == 0) return CRISPY_NS_OK;
   if (int rc = rows_prepare(b)) return rc;

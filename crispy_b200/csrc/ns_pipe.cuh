@@ -117,6 +117,9 @@ NS_DEV void hp_copy_rows(const float *src, long long src_stride, float *dst, lon
   }
 }
 
+// F32 (CRISPY_NS_BIQUAD_F32): the recursion in f32 arithmetic alone, every product and sum rounded to f32 --
+//   mem0 = mem1 + (b0 x - a0 y), mem1 = b1 x - a1 y -- the form a port that widens nothing would compute.
+template <bool F32 = false>
 NS_DEV void highpass_body(const Params &p, HpSmem &sm) {
   const int tid = Simt::tid();
   const int lane = tid & 31, warp = tid >> 5;
@@ -185,11 +188,17 @@ NS_DEV void highpass_body(const Params &p, HpSmem &sm) {
           for (int i = 0; i < 4; i++) {
             const float xi = x[i];
             const float yi = xi + m0;
-            const double xd = (double)xi, yd = (double)yi;
-            // a0*y and a1*y are exact in f64 (24 x 24 bit), so the fused forms round exactly like
-            // upstream's  mem1 + (b0*x - a0*y)  and  b1*x - a1*y
-            m0 = (float)((double)m1 + fma(na0, yd, -2.0 * xd));
-            m1 = (float)fma(na1, yd, xd);
+            if constexpr (F32) {
+              const float b0 = -2.f, b1 = 1.f, a0 = -1.99599f, a1 = .99600f;
+              m0 = m1 + (b0 * xi - a0 * yi);
+              m1 = b1 * xi - a1 * yi;
+            } else {
+              const double xd = (double)xi, yd = (double)yi;
+              // a0*y and a1*y are exact in f64 (24 x 24 bit), so the fused forms round exactly like
+              // upstream's  mem1 + (b0*x - a0*y)  and  b1*x - a1*y
+              m0 = (float)((double)m1 + fma(na0, yd, -2.0 * xd));
+              m1 = (float)fma(na1, yd, xd);
+            }
             y[i] = yi;
           }
           *reinterpret_cast<f4 *>(row + c) = f4{y[0], y[1], y[2], y[3]};
@@ -565,7 +574,8 @@ NS_DEV void highpass_par_body(const Params &p, HpParSmem &sm) {
 
 // =================================================================================================
 // K1: pitch analysis of R consecutive frames of one stream.  Every sum below is accumulated in the
-// oracle's order (ascending index, rounded product then rounded add), one lane per sum.
+// oracle's order (ascending index, rounded product then rounded add), one lane per sum; under sum policies
+// 1 and 2 the inner products the oracle sums as dot4 are split into four partial sums (Acc4).
 // =================================================================================================
 template <int R>
 struct PitchSmem {
@@ -657,13 +667,35 @@ NS_DEV float pitch_gain_f(float xy, float xx, float yy) { return xy / sqrtf(1.f 
 #endif
 #define NS_PRAGMA(x) _Pragma(#x)
 #define NS_UNROLL(n) NS_PRAGMA(unroll n)
-template <int N>
+// The chain of adds of one inner product, fed tap j as add(j & 3, x[j] y[j]) with j ascending from 0.  D4 = false:
+// one accumulator in ascending j (xiph's celt_inner_prod / xcorr_kernel, sum policy 0).  D4 = true: four partial sums
+// s[j & 3] reduced as ((s0 + s1) + s2) + s3 -- the oracle's dot4 (rnnoise_oracle.c, sum policies 1 and 2).  Every
+// length summed here is a multiple of 4, so dot4's sequential tail never runs.
+template <bool D4>
+struct Acc4 {
+  float s = 0.f;
+  NS_DEV void add(int, float v) { s += v; }
+  NS_DEV float sum() const { return s; }
+};
+template <>
+struct Acc4<true> {
+  float s[4] = {0.f, 0.f, 0.f, 0.f};
+  NS_DEV void add(int t, float v) { s[t] += v; }
+  NS_DEV float sum() const { return ((s[0] + s[1]) + s[2]) + s[3]; }
+};
+// K1's summation policy (CRISPY_NS_SUM_*): which of its inner products are summed as dot4
+template <int SP>
+constexpr bool kSpDot4 = SP >= 1;  // celt_inner_prod / dual_inner_prod
+template <int SP>
+constexpr bool kSpDot4Xcorr = SP >= 2;  // celt_pitch_xcorr (coarse search, autocorrelation)
+
+template <int N, bool D4 = false>
 NS_DEV float dot_shifted(const float *x, const float *yrow, int yoff) {
   static_assert(N % 4 == 0, "whole float4s");
   const float *ya = yrow + (yoff & ~3);
   const bool p1 = (yoff & 1) != 0, p2 = (yoff & 2) != 0;
   f4 lo = ld4(ya), hi = ld4(ya + 4), xv = ld4(x);
-  float sum = 0.f;
+  Acc4<D4> sum;
   NS_UNROLL(NS_DOT_UNROLL)
   for (int j = 0; j < N; j += 4) {
     // the next trip's operands are requested before this trip's chain of adds (the over-read of the
@@ -672,34 +704,34 @@ NS_DEV float dot_shifted(const float *x, const float *yrow, int yoff) {
     const float a0 = p1 ? lo.y : lo.x, a1 = p1 ? lo.z : lo.y, a2 = p1 ? lo.w : lo.z, a3 = p1 ? hi.x : lo.w,
                 a4 = p1 ? hi.y : hi.x, a5 = p1 ? hi.z : hi.y;
     const float y0 = p2 ? a2 : a0, y1 = p2 ? a3 : a1, y2 = p2 ? a4 : a2, y3 = p2 ? a5 : a3;
-    sum += xv.x * y0;
-    sum += xv.y * y1;
-    sum += xv.z * y2;
-    sum += xv.w * y3;
+    sum.add(0, xv.x * y0);
+    sum.add(1, xv.y * y1);
+    sum.add(2, xv.z * y2);
+    sum.add(3, xv.w * y3);
     lo = hi;
     hi = hi_n;
     xv = xv_n;
   }
-  return sum;
+  return sum.sum();
 }
 // the same with the shift S = (y - ya) known at compile time: no selects (used where a whole warp shares it)
-template <int N, int S>
+template <int N, int S, bool D4 = false>
 NS_DEV float dot_fixed_shift(const float *x, const float *ya) {
   f4 lo = ld4(ya), hi = ld4(ya + 4), xv = ld4(x);
-  float sum = 0.f;
+  Acc4<D4> sum;
   NS_UNROLL(NS_DOT_UNROLL)
   for (int j = 0; j < N; j += 4) {
     const f4 hi_n = ld4(ya + j + 8), xv_n = ld4(x + j + 4);
     const float w[8] = {lo.x, lo.y, lo.z, lo.w, hi.x, hi.y, hi.z, hi.w};
-    sum += xv.x * w[S];
-    sum += xv.y * w[S + 1];
-    sum += xv.z * w[S + 2];
-    sum += xv.w * w[S + 3];
+    sum.add(0, xv.x * w[S]);
+    sum.add(1, xv.y * w[S + 1]);
+    sum.add(2, xv.z * w[S + 2]);
+    sum.add(3, xv.w * w[S + 3]);
     lo = hi;
     hi = hi_n;
     xv = xv_n;
   }
-  return sum;
+  return sum.sum();
 }
 // three inner products at once for the consecutive lags whose windows start at ya + S, ya + S + 1 and
 // ya + S + 2: one pass over x and one stream of y feed three independent chains of adds
@@ -736,12 +768,12 @@ NS_DEV void dot3_fixed_shift(const float *x, const float *ya, float &s0, float &
 // taps needs come out of a two-level select network (shift by one, then by two) over the twelve loaded floats.
 // Fourteen selects per four taps buy full lanes: with compile-time shifts a warp only holds the items of one
 // alignment bucket (a quarter of a CTA's ~56 triples per warp-pass, seven active lanes on average).
-template <int N>
+template <int N, bool D4 = false>
 NS_DEV void dot3_shifted(const float *x, const float *yrow, int yoff, float &s0, float &s1, float &s2) {
   const float *ya = yrow + (yoff & ~3);
   const bool p1 = (yoff & 1) != 0, p2 = (yoff & 2) != 0;
   f4 w0 = ld4(ya), w1 = ld4(ya + 4), w2 = ld4(ya + 8), xv = ld4(x);
-  float a0 = 0.f, a1 = 0.f, a2 = 0.f;
+  Acc4<D4> a2, a1, a0;  // this order keeps the sequential instantiation's SASS what it was before Acc4
   NS_UNROLL(NS_DOT_UNROLL)
   for (int j = 0; j < N; j += 4) {
     const f4 w2_n = ld4(ya + j + 12), xv_n = ld4(x + j + 4);
@@ -750,28 +782,29 @@ NS_DEV void dot3_shifted(const float *x, const float *yrow, int yoff, float &s0,
                 b4 = p1 ? w1.y : w1.x, b5 = p1 ? w1.z : w1.y, b6 = p1 ? w1.w : w1.z, b7 = p1 ? w2.x : w1.w;
     const float y0 = p2 ? b2 : b0, y1 = p2 ? b3 : b1, y2 = p2 ? b4 : b2, y3 = p2 ? b5 : b3, y4 = p2 ? b6 : b4,
                 y5 = p2 ? b7 : b5;
-    a0 += xv.x * y0;
-    a1 += xv.x * y1;
-    a2 += xv.x * y2;
-    a0 += xv.y * y1;
-    a1 += xv.y * y2;
-    a2 += xv.y * y3;
-    a0 += xv.z * y2;
-    a1 += xv.z * y3;
-    a2 += xv.z * y4;
-    a0 += xv.w * y3;
-    a1 += xv.w * y4;
-    a2 += xv.w * y5;
+    a0.add(0, xv.x * y0);
+    a1.add(0, xv.x * y1);
+    a2.add(0, xv.x * y2);
+    a0.add(1, xv.y * y1);
+    a1.add(1, xv.y * y2);
+    a2.add(1, xv.y * y3);
+    a0.add(2, xv.z * y2);
+    a1.add(2, xv.z * y3);
+    a2.add(2, xv.z * y4);
+    a0.add(3, xv.w * y3);
+    a1.add(3, xv.w * y4);
+    a2.add(3, xv.w * y5);
     w0 = w1;
     w1 = w2;
     w2 = w2_n;
     xv = xv_n;
   }
-  s0 = a0;
-  s1 = a1;
-  s2 = a2;
+  s0 = a0.sum();
+  s1 = a1.sum();
+  s2 = a2.sum();
 }
-NS_DEV float dot480_shifted(const float *row, int yoff) { return dot_shifted<480>(row + 384, row, yoff); }
+template <bool D4 = false>
+NS_DEV float dot480_shifted(const float *row, int yoff) { return dot_shifted<480, D4>(row + 384, row, yoff); }
 
 // find_best_pitch's running energy: out[i] = Syy before lag i, Syy <- max(1, Syy + y[i+len]^2 - y[i]^2), for
 // i < n (rounded up to 4).  y, out 16-byte aligned; out may alias y[0..n) (each y[i] is read before out[i]
@@ -829,7 +862,8 @@ __device__ unsigned long long g_pitch_phase_cycles[24];
 #define NS_PHASE_BEGIN() do {} while (0)
 #define NS_PHASE_MARK(i) do {} while (0)
 #endif
-template <int R, int NT>
+// SP: the summation policy (CRISPY_NS_SUM_*, kSpDot4 / kSpDot4Xcorr above); 0 is xiph's sequential order
+template <int R, int NT, int SP = 0>
 NS_DEV void pitch_body(const Params &p, PitchSmem<R> &sm) {
   const int tid = Simt::tid();
   NS_PHASE_BEGIN();
@@ -879,21 +913,21 @@ NS_DEV void pitch_body(const Params &p, PitchSmem<R> &sm) {
         const float *y = x + k;
         f4 xv = ld4(x);
         float y0 = y[0], y1 = y[1], y2 = y[2], y3 = y[3];
-        float sum = 0.f;
+        Acc4<kSpDot4Xcorr<SP>> sum;
         NS_UNROLL(NS_DOT_UNROLL)
         for (int i = 0; i < kLpLen - 4; i += 4) {  // the last trip's over-read stays inside the padded row
           const f4 xn = ld4(x + i + 4);
           const float n0 = y[i + 4], n1 = y[i + 5], n2 = y[i + 6], n3 = y[i + 7];
-          sum += xv.x * y0;
-          sum += xv.y * y1;
-          sum += xv.z * y2;
-          sum += xv.w * y3;
+          sum.add(0, xv.x * y0);
+          sum.add(1, xv.y * y1);
+          sum.add(2, xv.z * y2);
+          sum.add(3, xv.w * y3);
           xv = xn;
           y0 = n0, y1 = n1, y2 = n2, y3 = n3;
         }
         float d = 0.f;
         for (int i = k + kLpLen - 4; i < kLpLen; i++) d += x[i] * x[i - k];
-        sm.ac[f][k] = sum + d;
+        sm.ac[f][k] = sum.sum() + d;
       }
     }
   } else if (NT >= 5 * 32 && R <= 32) {
@@ -902,11 +936,11 @@ NS_DEV void pitch_body(const Params &p, PitchSmem<R> &sm) {
       const float *x = sm.xr + f * kLpStride;
       float sum;
       switch (k) {
-        case 0: sum = dot_fixed_shift<kLpLen - 4, 0>(x, x); break;
-        case 1: sum = dot_fixed_shift<kLpLen - 4, 1>(x, x); break;
-        case 2: sum = dot_fixed_shift<kLpLen - 4, 2>(x, x); break;
-        case 3: sum = dot_fixed_shift<kLpLen - 4, 3>(x, x); break;
-        default: sum = dot_fixed_shift<kLpLen - 4, 0>(x, x + 4); break;
+        case 0: sum = dot_fixed_shift<kLpLen - 4, 0, kSpDot4Xcorr<SP>>(x, x); break;
+        case 1: sum = dot_fixed_shift<kLpLen - 4, 1, kSpDot4Xcorr<SP>>(x, x); break;
+        case 2: sum = dot_fixed_shift<kLpLen - 4, 2, kSpDot4Xcorr<SP>>(x, x); break;
+        case 3: sum = dot_fixed_shift<kLpLen - 4, 3, kSpDot4Xcorr<SP>>(x, x); break;
+        default: sum = dot_fixed_shift<kLpLen - 4, 0, kSpDot4Xcorr<SP>>(x, x + 4); break;
       }
       float d = 0.f;
       for (int i = k + kLpLen - 4; i < kLpLen; i++) d += x[i] * x[i - k];
@@ -916,7 +950,7 @@ NS_DEV void pitch_body(const Params &p, PitchSmem<R> &sm) {
     for (int it = tid; it < nfr * 5; it += NT) {
       const int f = it / 5, k = it - f * 5;
       const float *x = sm.xr + f * kLpStride;
-      const float sum = dot_shifted<kLpLen - 4>(x, x, k);
+      const float sum = dot_shifted<kLpLen - 4, kSpDot4Xcorr<SP>>(x, x, k);
       float d = 0.f;
       for (int i = k + kLpLen - 4; i < kLpLen; i++) d += x[i] * x[i - k];
       sm.ac[f][k] = sum + d;
@@ -1007,6 +1041,7 @@ NS_DEV void pitch_body(const Params &p, PitchSmem<R> &sm) {
   const int chain_lane = tid & 31;
   const bool chain_b = (tid >> 5) == NW - 2 && chain_lane < nfr, chain_c = (tid >> 5) == NW - 3 && chain_lane < nfr;
   float ch_acc = chain_b ? 1.f : 0.f;
+  float ch_p1 = 0.f, ch_p2 = 0.f, ch_p3 = 0.f;  // chain C's partial sums of taps j = 1, 2, 3 (mod 4) under dot4
   int ch_blk = 0;  // blocks done: 30 for the sum of squares, then 19 (B) / 24 (C) for the recurrence
   auto chain_run = [&](int budget, bool recur_b) {
     if (!chain_b && !chain_c) return;
@@ -1015,10 +1050,21 @@ NS_DEV void pitch_body(const Params &p, PitchSmem<R> &sm) {
     for (; budget > 0 && ch_blk < 30; budget--, ch_blk++) {
       const float *q = y + 16 * ch_blk;
       const f4 v0 = ld4(q), v1 = ld4(q + 4), v2 = ld4(q + 8), v3 = ld4(q + 12);
-      ch_acc += v0.x * v0.x, ch_acc += v0.y * v0.y, ch_acc += v0.z * v0.z, ch_acc += v0.w * v0.w;
-      ch_acc += v1.x * v1.x, ch_acc += v1.y * v1.y, ch_acc += v1.z * v1.z, ch_acc += v1.w * v1.w;
-      ch_acc += v2.x * v2.x, ch_acc += v2.y * v2.y, ch_acc += v2.z * v2.z, ch_acc += v2.w * v2.w;
-      ch_acc += v3.x * v3.x, ch_acc += v3.y * v3.y, ch_acc += v3.z * v3.z, ch_acc += v3.w * v3.w;
+      if constexpr (kSpDot4<SP>) {
+        if (chain_c) {  // xx is dual_inner_prod's: dot4 (chain B's Syy belongs to find_best_pitch and stays sequential)
+          ch_acc += v0.x * v0.x, ch_p1 += v0.y * v0.y, ch_p2 += v0.z * v0.z, ch_p3 += v0.w * v0.w;
+          ch_acc += v1.x * v1.x, ch_p1 += v1.y * v1.y, ch_p2 += v1.z * v1.z, ch_p3 += v1.w * v1.w;
+          ch_acc += v2.x * v2.x, ch_p1 += v2.y * v2.y, ch_p2 += v2.z * v2.z, ch_p3 += v2.w * v2.w;
+          ch_acc += v3.x * v3.x, ch_p1 += v3.y * v3.y, ch_p2 += v3.z * v3.z, ch_p3 += v3.w * v3.w;
+          if (ch_blk == 29) ch_acc = ((ch_acc + ch_p1) + ch_p2) + ch_p3;
+        }
+      }
+      if (!kSpDot4<SP> || !chain_c) {
+        ch_acc += v0.x * v0.x, ch_acc += v0.y * v0.y, ch_acc += v0.z * v0.z, ch_acc += v0.w * v0.w;
+        ch_acc += v1.x * v1.x, ch_acc += v1.y * v1.y, ch_acc += v1.z * v1.z, ch_acc += v1.w * v1.w;
+        ch_acc += v2.x * v2.x, ch_acc += v2.y * v2.y, ch_acc += v2.z * v2.z, ch_acc += v2.w * v2.w;
+        ch_acc += v3.x * v3.x, ch_acc += v3.y * v3.y, ch_acc += v3.z * v3.z, ch_acc += v3.w * v3.w;
+      }
       if (ch_blk == 29 && chain_c) {
         sm.xx[f] = ch_acc;
         sm.xr[f * kLpStride + 432] = ch_acc;  // yy_lookup[0]
@@ -1076,14 +1122,15 @@ NS_DEV void pitch_body(const Params &p, PitchSmem<R> &sm) {
       syy_recurrence(sumsq_from<240>(1.f, y4), y4, 240, 147, sm.sb6[l]);
     }
   }
-  for (int it = tid; it < nfr * 19; it += NT) {  // eight lags per lane: one new float4 of y and one of x feed 32 MACs
-    const int f = it / 19, q = it - f * 19;
+  // Under dot4 a lag holds four partial sums: four lags per lane keep the accumulators at sixteen registers.
+  constexpr bool kD4x = kSpDot4Xcorr<SP>;
+  constexpr int kLpl = kD4x ? 4 : 8, kQpf = 152 / kLpl;  // lags per lane, lanes per frame
+  for (int it = tid; it < nfr * kQpf; it += NT) {  // eight lags per lane: one new float4 of y and one of x feed 32 MACs
+    const int f = it / kQpf, q = it - f * kQpf;
     const float *y4 = sm.xr + f * kLpStride;
     const float *x4 = y4 + 192;
-    const float *yb = y4 + 8 * q;
-    float a[8];
-#pragma unroll
-    for (int l = 0; l < 8; l++) a[l] = 0.f;
+    const float *yb = y4 + kLpl * q;
+    Acc4<kD4x> a[kLpl];
     f4 w0 = ld4(yb), w1 = ld4(yb + 4);
 #pragma unroll 2
     for (int j = 0; j < 240; j += 4) {
@@ -1093,13 +1140,14 @@ NS_DEV void pitch_body(const Params &p, PitchSmem<R> &sm) {
 #pragma unroll
       for (int t = 0; t < 4; t++)
 #pragma unroll
-        for (int l = 0; l < 8; l++) a[l] += xt[t] * w[l + t];
+        for (int l = 0; l < kLpl; l++) a[l].add(t, xt[t] * w[l + t]);
       w0 = w1;
       w1 = w2;
     }
-    float *dst = sm.xc[f] + 8 * q;
-    *reinterpret_cast<f4 *>(dst) = f4{a[0], a[1], a[2], a[3]};
-    *reinterpret_cast<f4 *>(dst + 4) = f4{a[4], a[5], a[6], a[7]};
+    float *dst = sm.xc[f] + kLpl * q;
+#pragma unroll
+    for (int l = 0; l < kLpl; l += 4)
+      *reinterpret_cast<f4 *>(dst + l) = f4{a[l].sum(), a[l + 1].sum(), a[l + 2].sum(), a[l + 3].sum()};
   }
   chain_run(25, false);
   Simt::cta_sync();
@@ -1229,7 +1277,7 @@ NS_DEV void pitch_body(const Params &p, PitchSmem<R> &sm) {
     const int dd = i - c0;
     const bool ok = (i >= 0) && (i < 294) && (c < 5 || dd > 2 || dd < -2);
     float sum = 0.f;
-    if (ok) sum = dot480_shifted(lp, i);
+    if (ok) sum = dot480_shifted<kSpDot4<SP>>(lp, i);
     sm.fi[f][c] = ok ? i : -1;
     sm.fx[f][c] = sum < -1.f ? -1.f : sum;
   }
@@ -1317,7 +1365,7 @@ NS_DEV void pitch_body(const Params &p, PitchSmem<R> &sm) {
           const int f = e & 31, Tc = (e >> 5) & 0x1FF, k = e >> 14;
           const float *row = sm.xlp + f * kLpStride;
           float sp, sc, sm1;  // lags Tc+1, Tc, Tc-1
-          dot3_shifted<480>(row + 384, row, 384 - Tc - 1, sp, sc, sm1);
+          dot3_shifted<480, kSpDot4<SP>>(row + 384, row, 384 - Tc - 1, sp, sc, sm1);
           const int d = 2 + 4 * (k - 2);
           sm.dots[f][k == 1 ? 0 : d] = sm1;
           sm.dots[f][k == 1 ? kDotXy0 : d + 1] = sc;
@@ -1329,7 +1377,7 @@ NS_DEV void pitch_body(const Params &p, PitchSmem<R> &sm) {
           const int e = (&sm.sgl[0][0])[it];
           const int f = e & 31, lag = (e >> 5) & 0x1FF, k = e >> 14;
           const float *row = sm.xlp + f * kLpStride;
-          sm.dots[f][2 + 4 * (k - 2) + 3] = dot_shifted<480>(row + 384, row, 384 - lag);
+          sm.dots[f][2 + 4 * (k - 2) + 3] = dot_shifted<480, kSpDot4<SP>>(row + 384, row, 384 - lag);
         }
       }
     }

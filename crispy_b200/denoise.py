@@ -51,6 +51,17 @@ class Model:
         check(_lib.lib().crispy_ns_model_from_bytes(blob, len(blob), C.byref(h)))
         return cls(h.value)
 
+    @property
+    def numerics(self) -> int:
+        """Which float32 arithmetic the pitch path's decisions follow: a SUM_* order | BIQUAD_F32 (crispy_b200._lib;
+        include/crispy_ns.h crispy_ns_model_set_numerics).  0, the default, is xiph's C.  Handles copy it when they are
+        created; to_bytes / from_bytes do not carry it."""
+        return int(_lib.lib().crispy_ns_model_numerics(self._h))
+
+    @numerics.setter
+    def numerics(self, value: int) -> None:
+        check(_lib.lib().crispy_ns_model_set_numerics(self._h, int(value)))
+
     def to_bytes(self) -> bytes:
         n = C.c_size_t()
         check(_lib.lib().crispy_ns_model_to_bytes(self._h, None, 0, C.byref(n)))

@@ -80,6 +80,32 @@ int crispy_ns_model_from_bytes(const void *blob, size_t len, crispy_ns_model **o
 int crispy_ns_model_to_bytes(const crispy_ns_model *m, void *buf, size_t cap, size_t *needed);
 void crispy_ns_model_destroy(crispy_ns_model *m);
 
+/* ---- numerics: which float32 arithmetic the pitch path's discrete decisions follow.  The product reproduces one
+ * arithmetic bit for bit; which one nnnoiseless itself computes is not pinned (DESIGN.md section 6, points 1 and 4), so
+ * the alternatives are a setting of the model, the object that names the reference being matched.
+ *   sum order (CRISPY_NS_SUM_MASK): the inner products of pitch_search / remove_doubling (celt_inner_prod,
+ *     dual_inner_prod) and the cross-correlations (celt_pitch_xcorr: coarse search, autocorrelation) summed in xiph's
+ *     sequential order (0, the default), as four interleaved partial sums ((s0 + s1) + s2) + s3 in the inner products
+ *     only (DOT4), or in the cross-correlations as well (DOT4_XCORR);
+ *   CRISPY_NS_BIQUAD_F32: the high-pass biquad in f32 arithmetic, every product and sum rounded separately, instead
+ *     of f32 state with f64 intermediates as the C computes it.
+ * Every handle copies the model's setting when it is created (crispy_ns_create, _batch_create, _multi_create,
+ * _denoise_wav_files); changing the model later does not affect it; model == NULL means 0.  The CRNSMDL1 blob does not
+ * carry the setting: crispy_ns_model_to_bytes / _from_bytes leave it out, and a model from bytes starts at 0.
+ * set_numerics returns CRISPY_NS_EINVAL for a null model, unknown bits or sum order 3.  Builds whose pitch kernel
+ * knows only the sequential order (-DNS_PITCH_V7) refuse a nonzero sum order at handle creation (CRISPY_NS_EINVAL).
+ * A stream record (crispy_ns_batch_save_streams) carries the batch's numerics; a whole-batch state
+ * (crispy_ns_batch_save_state) does not, and is only meaningful in a batch of the same numerics. ---- */
+enum {
+  CRISPY_NS_SUM_SEQUENTIAL = 0u, /* xiph order: the default */
+  CRISPY_NS_SUM_DOT4 = 1u,       /* four partial sums in celt_inner_prod / dual_inner_prod */
+  CRISPY_NS_SUM_DOT4_XCORR = 2u, /* DOT4, and in celt_pitch_xcorr as well */
+  CRISPY_NS_SUM_MASK = 3u,
+  CRISPY_NS_BIQUAD_F32 = 1u << 4 /* biquad in f32 arithmetic, no f64 intermediates, no contraction */
+};
+int crispy_ns_model_set_numerics(crispy_ns_model *m, uint32_t numerics);
+uint32_t crispy_ns_model_numerics(const crispy_ns_model *m);
+
 /* ---- DenoiseState::new (audio.rs:229).  model == NULL selects the built-in default: the blob
  * named by $CRISPY_NS_WEIGHTS if set, else synthetic seed 0. ---- */
 int crispy_ns_create(const crispy_ns_model *model, int device, crispy_ns_state **out);
@@ -117,7 +143,8 @@ int crispy_ns_process_streams_debug(crispy_ns_batch *b, const void *d_in, void *
                                     uint32_t flags, float volume, void *cuda_stream);
 int crispy_ns_debug_floats(void);
 
-/* checkpoint / resume of every stream's DenoiseState (host buffers) */
+/* checkpoint / resume of every stream's DenoiseState (host buffers); the state does not record the batch's numerics
+ * and is only meaningful when loaded into a batch of the same numerics */
 size_t crispy_ns_batch_state_size(const crispy_ns_batch *b);
 int crispy_ns_batch_save_state(crispy_ns_batch *b, void *buf, size_t len);
 int crispy_ns_batch_load_state(crispy_ns_batch *b, const void *buf, size_t len);
@@ -153,8 +180,9 @@ int crispy_ns_process_streams_subset_host(crispy_ns_batch *b, const int *streams
  * every call already enqueued, and before the batch's next call; cuda_stream waits for it */
 int crispy_ns_batch_reset_streams(crispy_ns_batch *b, const int *streams, int n, void *cuda_stream);
 /* one self-describing record per listed stream (host buffers, synchronous): a 16-byte header ("CRNSSTR1", the state's
- * float count, 0) and the stream's DenoiseState -- 11,152 bytes in this build.  A record loads into any stream of
- * any batch of this build; save_streams needs len >= n records, load_streams exactly n records. */
+ * float count, the batch's numerics) and the stream's DenoiseState -- 11,152 bytes in this build.  A record loads into
+ * any stream of any batch of this build with the same numerics (else CRISPY_NS_EINVAL); save_streams needs len >= n
+ * records, load_streams exactly n records. */
 size_t crispy_ns_stream_state_size(void);
 int crispy_ns_batch_save_streams(crispy_ns_batch *b, const int *streams, int n, void *buf, size_t len);
 int crispy_ns_batch_load_streams(crispy_ns_batch *b, const int *streams, int n, const void *buf, size_t len);

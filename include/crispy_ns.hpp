@@ -109,6 +109,9 @@ class Model {
     detail::check(crispy_ns_model_to_bytes(h_, b.data(), b.size(), &n));
     return b;
   }
+  // CRISPY_NS_SUM_* | CRISPY_NS_BIQUAD_F32 (crispy_ns.h): the arithmetic the handles created from this model follow
+  void set_numerics(std::uint32_t numerics) { detail::check(crispy_ns_model_set_numerics(h_, numerics)); }
+  std::uint32_t numerics() const { return crispy_ns_model_numerics(h_); }
   Model(Model &&o) noexcept : h_(std::exchange(o.h_, nullptr)) {}
   Model &operator=(Model &&o) noexcept {
     if (this != &o) {
