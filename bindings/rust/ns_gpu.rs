@@ -49,6 +49,21 @@ pub const CRISPY_NS_SUM_DOT4_XCORR: u32 = 2;
 pub const CRISPY_NS_SUM_MASK: u32 = 3;
 pub const CRISPY_NS_BIQUAD_F32: u32 = 1 << 4;
 
+/// crispy_ns_controls: per-stream attenuation limit and voice gate with hold (include/crispy_ns.h).  `Default` (all
+/// zero) is off.  Out-of-range or NaN values are refused with an error and change nothing.
+#[repr(C)]
+#[derive(Clone, Copy, Debug, Default, PartialEq)]
+pub struct Controls {
+    /// [0, 1]; floor on every band gain applied to the spectrum; 0 = no limit
+    pub min_gain: f32,
+    /// [0, 1]; a frame is voiced if its VAD >= threshold; 0 = gate off
+    pub gate_threshold: f32,
+    /// [0, 1 << 20] frames the gate stays open after the last voiced frame
+    pub gate_hold: i32,
+    /// [0, 1]; output gain while the gate is closed; 0 = mute
+    pub gate_gain: f32,
+}
+
 extern "C" {
     fn crispy_ns_last_error() -> *const c_char;
     fn crispy_ns_device_count() -> c_int;
@@ -72,6 +87,14 @@ extern "C" {
         app_stride: i64, flags: u32, volume: c_float,
     ) -> c_int;
     fn crispy_ns_batch_reset_streams(b: *mut CrispyNsBatch, streams: *const c_int, n: c_int, cuda_stream: *mut c_void) -> c_int;
+    // controls / out: arrays of `Controls`
+    fn crispy_ns_batch_set_controls(b: *mut CrispyNsBatch, streams: *const c_int, n: c_int, controls: *const c_void,
+                                    cuda_stream: *mut c_void) -> c_int;
+    fn crispy_ns_batch_get_controls(b: *mut CrispyNsBatch, streams: *const c_int, n: c_int, out: *mut c_void) -> c_int;
+    fn crispy_ns_set_controls(st: *mut CrispyNsState, controls: *const c_void) -> c_int;
+    fn crispy_ns_get_controls(st: *mut CrispyNsState, out: *mut c_void) -> c_int;
+    fn crispy_ns_multi_set_controls(m: *mut CrispyNsMulti, streams: *const c_int, n: c_int, controls: *const c_void) -> c_int;
+    fn crispy_ns_multi_get_controls(m: *mut CrispyNsMulti, streams: *const c_int, n: c_int, out: *mut c_void) -> c_int;
     fn crispy_ns_stream_state_size() -> usize;
     fn crispy_ns_batch_save_streams(b: *mut CrispyNsBatch, streams: *const c_int, n: c_int, buf: *mut c_void, len: usize) -> c_int;
     fn crispy_ns_batch_load_streams(b: *mut CrispyNsBatch, streams: *const c_int, n: c_int, buf: *const c_void, len: usize)
@@ -143,6 +166,16 @@ impl<'model> DenoiseState<'model> {
     pub fn reset(&mut self) {
         let rc = unsafe { crispy_ns_reset(self.h) };
         assert!(rc == 0, "crispy_ns_reset failed: {}", last_error());
+    }
+    /// attenuation limit and voice gate of this stream, from its next frame on; a reset turns them off
+    pub fn set_controls(&mut self, c: &Controls) -> Result<(), String> {
+        let rc = unsafe { crispy_ns_set_controls(self.h, c as *const Controls as *const c_void) };
+        if rc == 0 { Ok(()) } else { Err(last_error()) }
+    }
+    pub fn controls(&mut self) -> Result<Controls, String> {
+        let mut c = Controls::default();
+        let rc = unsafe { crispy_ns_get_controls(self.h, &mut c as *mut Controls as *mut c_void) };
+        if rc == 0 { Ok(c) } else { Err(last_error()) }
     }
 }
 impl<'model> Drop for DenoiseState<'model> {
@@ -256,6 +289,20 @@ impl BatchDenoiser {
         }
         Ok(())
     }
+    /// `controls[i]` for `streams[i]`, ordered before the next call; stream records carry them, resets turn them off
+    pub fn set_controls(&mut self, streams: &[i32], controls: &[Controls]) -> Result<(), String> {
+        assert_eq!(streams.len(), controls.len());
+        let rc = unsafe {
+            crispy_ns_batch_set_controls(self.h, streams.as_ptr(), streams.len() as c_int, controls.as_ptr() as *const c_void,
+                                         std::ptr::null_mut())
+        };
+        if rc == 0 { Ok(()) } else { Err(last_error()) }
+    }
+    pub fn controls(&mut self, streams: &[i32]) -> Result<Vec<Controls>, String> {
+        let mut c = vec![Controls::default(); streams.len()];
+        let rc = unsafe { crispy_ns_batch_get_controls(self.h, streams.as_ptr(), streams.len() as c_int, c.as_mut_ptr() as *mut c_void) };
+        if rc == 0 { Ok(c) } else { Err(last_error()) }
+    }
     /// one self-describing record per listed stream; it loads into any stream of any batch of this build
     pub fn save_streams(&mut self, streams: &[i32]) -> Result<Vec<u8>, String> {
         let n = streams.len() * unsafe { crispy_ns_stream_state_size() };
@@ -312,6 +359,17 @@ impl MultiDenoiser {
                                                  stride as i64, 0, 0, CRISPY_NS_IN_I16 | CRISPY_NS_OUT_I16, 1.0)
         };
         if rc == 0 { Ok(()) } else { Err(last_error()) }
+    }
+    /// as BatchDenoiser::set_controls over the handle's global stream ids
+    pub fn set_controls(&mut self, streams: &[i32], controls: &[Controls]) -> Result<(), String> {
+        assert_eq!(streams.len(), controls.len());
+        let rc = unsafe { crispy_ns_multi_set_controls(self.h, streams.as_ptr(), streams.len() as c_int, controls.as_ptr() as *const c_void) };
+        if rc == 0 { Ok(()) } else { Err(last_error()) }
+    }
+    pub fn controls(&mut self, streams: &[i32]) -> Result<Vec<Controls>, String> {
+        let mut c = vec![Controls::default(); streams.len()];
+        let rc = unsafe { crispy_ns_multi_get_controls(self.h, streams.as_ptr(), streams.len() as c_int, c.as_mut_ptr() as *mut c_void) };
+        if rc == 0 { Ok(c) } else { Err(last_error()) }
     }
 }
 impl Drop for MultiDenoiser {

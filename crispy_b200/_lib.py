@@ -43,7 +43,15 @@ SYMBOLS = [
     "crispy_ns_process_streams_subset", "crispy_ns_process_streams_subset_host", "crispy_ns_batch_reset_streams",
     "crispy_ns_stream_state_size", "crispy_ns_batch_save_streams", "crispy_ns_batch_load_streams",
     "crispy_ns_model_set_numerics", "crispy_ns_model_numerics",
+    "crispy_ns_batch_set_controls", "crispy_ns_batch_get_controls", "crispy_ns_set_controls", "crispy_ns_get_controls",
+    "crispy_ns_multi_set_controls", "crispy_ns_multi_get_controls",
 ]
+
+
+class Controls(C.Structure):
+    """crispy_ns_controls (include/crispy_ns.h): per-stream attenuation limit and voice gate; all zero = off"""
+    _fields_ = [("min_gain", C.c_float), ("gate_threshold", C.c_float), ("gate_hold", C.c_int32),
+                ("gate_gain", C.c_float)]
 
 
 class CrispyNsError(RuntimeError):
@@ -99,6 +107,13 @@ def lib() -> C.CDLL:
     L.crispy_ns_stream_state_size.restype = C.c_size_t
     L.crispy_ns_batch_save_streams.argtypes = [vp, ip, C.c_int, vp, C.c_size_t]
     L.crispy_ns_batch_load_streams.argtypes = [vp, ip, C.c_int, vp, C.c_size_t]
+    cp = C.POINTER(Controls)
+    L.crispy_ns_batch_set_controls.argtypes = [vp, ip, C.c_int, cp, vp]
+    L.crispy_ns_batch_get_controls.argtypes = [vp, ip, C.c_int, cp]
+    L.crispy_ns_set_controls.argtypes = [vp, cp]
+    L.crispy_ns_get_controls.argtypes = [vp, cp]
+    L.crispy_ns_multi_set_controls.argtypes = [vp, ip, C.c_int, cp]
+    L.crispy_ns_multi_get_controls.argtypes = [vp, ip, C.c_int, cp]
     L.crispy_ns_batch_info.argtypes = [vp, C.POINTER(C.c_int), C.POINTER(C.c_int), C.POINTER(i64), C.POINTER(i64)]
     L.crispy_ns_kernel_count.restype = C.c_int
     L.crispy_ns_kernel_name.argtypes = [C.c_int]

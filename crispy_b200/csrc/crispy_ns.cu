@@ -160,6 +160,24 @@ __global__ void __launch_bounds__(256) ns_state_rows_kernel(const __grid_constan
   }
 }
 
+// crispy_ns_batch_set_controls: thread j writes the four control words (ns_common.h kStCtl*) of state row ids[j]; the
+// gate's carry (left, previous G) is left alone, so new controls take effect from the next frame on
+constexpr int kCtlIds = 192;  // entries per launch: the parameter block stays under 4 KB
+struct ControlArgs {
+  float *state;
+  int n;
+  int ids[kCtlIds];
+  uint32_t words[kCtlIds][4];
+};
+__global__ void __launch_bounds__(kCtlIds) ns_set_controls_kernel(const __grid_constant__ ControlArgs a) {
+  const int j = threadIdx.x;
+  if (j >= a.n) return;
+  uint32_t *row = reinterpret_cast<uint32_t *>(a.state + (long long)a.ids[j] * ns::kStateFloats);
+  static_assert(ns::kStCtlGateThr == ns::kStCtlMinGain + 1 && ns::kStCtlGateHold == ns::kStCtlMinGain + 2 &&
+                    ns::kStCtlGateGain == ns::kStCtlMinGain + 3, "the four control words are contiguous");
+  for (int w = 0; w < 4; w++) row[ns::kStCtlMinGain + w] = a.words[j][w];
+}
+
 // a4/f2: out[s][n] = in[s][idx[n]-1] + (in[s][idx[n]] - in[s][idx[n]-1]) * frac[n], no FMA
 // contraction so the result is bit-identical to LinearResampler::process_sample (audio.rs:125-129).
 __global__ void __launch_bounds__(256) ns_linear_resample_kernel(const float *__restrict__ in, float *__restrict__ out,
@@ -1225,15 +1243,21 @@ static int check_ids(const crispy_ns_batch *b, const int *ids, int n, const char
   return CRISPY_NS_OK;
 }
 
-// d_rows and e_rows exist, and the internal streams are ordered after an asynchronous whole-batch reset
-static int rows_prepare(crispy_ns_batch *b) {
+// e_rows exists, and the internal streams are ordered after an asynchronous whole-batch reset
+static int rows_order(crispy_ns_batch *b) {
   NS_CUDA(cudaSetDevice(b->device));
-  if (!b->d_rows) NS_CUDA(cudaMalloc((void **)&b->d_rows, (size_t)b->n_streams * kRowBytes));
   if (!b->e_rows) NS_CUDA(cudaEventCreateWithFlags(&b->e_rows, cudaEventDisableTiming));
   if (b->reset_pending) {
     for (int k = 0; k < kNumKernels; k++) NS_CUDA(cudaStreamWaitEvent(b->s_k[k], b->e_reset, 0));
     b->reset_pending = false;
   }
+  return CRISPY_NS_OK;
+}
+
+// as rows_order, and d_rows exists
+static int rows_prepare(crispy_ns_batch *b) {
+  if (int rc = rows_order(b)) return rc;
+  if (!b->d_rows) NS_CUDA(cudaMalloc((void **)&b->d_rows, (size_t)b->n_streams * kRowBytes));
   return CRISPY_NS_OK;
 }
 
@@ -1388,6 +1412,68 @@ int batch_load_streams(crispy_ns_batch *b, const int *streams, int n, const void
   NS_CUDA(cudaStreamSynchronize(s6));  // buf may be reused as soon as the call returns
   return CRISPY_NS_OK;
 }
+// ---- per-stream suppression controls: four words of the state row (ns_common.h kStCtl*), so subset calls, stream
+// records, whole-batch states and the single-frame graphs carry them, and every reset turns them off
+static bool unit_interval(float x) { return x >= 0.f && x <= 1.f; }  // false for NaN
+static int check_controls(const crispy_ns_controls *c, int n, const char *what) {
+  if (n > 0 && !c) return fail(CRISPY_NS_EINVAL, std::string(what) + ": controls is null");
+  for (int i = 0; i < n; i++)
+    if (!unit_interval(c[i].min_gain) || !unit_interval(c[i].gate_threshold) || !unit_interval(c[i].gate_gain) ||
+        c[i].gate_hold < 0 || c[i].gate_hold > (1 << 20))
+      return fail(CRISPY_NS_EINVAL, std::string(what) + ": a control is out of range or NaN");
+  return CRISPY_NS_OK;
+}
+
+int batch_set_controls(crispy_ns_batch *b, const int *streams, int n, const void *controls_v, void *cuda_stream) {
+  const crispy_ns_controls *controls = static_cast<const crispy_ns_controls *>(controls_v);
+  if (int rc = check_ids(b, streams, n, "batch_set_controls")) return rc;
+  if (int rc = check_controls(controls, n, "batch_set_controls")) return rc;
+  if (n == 0) return CRISPY_NS_OK;
+  if (int rc = rows_order(b)) return rc;
+  cudaStream_t s6 = b->s_k[kNumKernels - 1];
+  NS_CUDA(cudaEventRecord(b->e_start, (cudaStream_t)cuda_stream));  // behind the caller's work, as reset_streams
+  NS_CUDA(cudaStreamWaitEvent(s6, b->e_start, 0));
+  ControlArgs a;
+  a.state = b->d_state;
+  for (int first = 0; first < n; first += kCtlIds) {
+    a.n = n - first < kCtlIds ? n - first : kCtlIds;
+    for (int j = 0; j < a.n; j++) {
+      const crispy_ns_controls &c = controls[first + j];
+      a.ids[j] = streams[first + j];
+      memcpy(&a.words[j][0], &c.min_gain, 4);
+      memcpy(&a.words[j][1], &c.gate_threshold, 4);
+      memcpy(&a.words[j][2], &c.gate_hold, 4);
+      memcpy(&a.words[j][3], &c.gate_gain, 4);
+    }
+    ns_set_controls_kernel<<<1, kCtlIds, 0, s6>>>(a);
+    NS_CUDA(cudaGetLastError());
+  }
+  if (int rc = rows_publish(b)) return rc;
+  NS_CUDA(cudaStreamWaitEvent((cudaStream_t)cuda_stream, b->e_rows, 0));
+  return CRISPY_NS_OK;
+}
+
+int batch_get_controls(crispy_ns_batch *b, const int *streams, int n, void *out_v) {
+  crispy_ns_controls *out = static_cast<crispy_ns_controls *>(out_v);
+  if (int rc = check_ids(b, streams, n, "batch_get_controls")) return rc;
+  if (n > 0 && !out) return fail(CRISPY_NS_EINVAL, "batch_get_controls: out is null");
+  if (n == 0) return CRISPY_NS_OK;
+  if (int rc = rows_order(b)) return rc;
+  cudaStream_t s6 = b->s_k[kNumKernels - 1];  // behind every set_controls, reset and load already enqueued
+  std::vector<uint32_t> w((size_t)b->n_streams * 4);
+  NS_CUDA(cudaMemcpy2DAsync(w.data(), 16, b->d_state + ns::kStCtlMinGain, kRowBytes, 16, (size_t)b->n_streams,
+                            cudaMemcpyDeviceToHost, s6));
+  NS_CUDA(cudaStreamSynchronize(s6));
+  for (int i = 0; i < n; i++) {
+    const uint32_t *r = &w[(size_t)streams[i] * 4];
+    memcpy(&out[i].min_gain, &r[0], 4);
+    memcpy(&out[i].gate_threshold, &r[1], 4);
+    memcpy(&out[i].gate_hold, &r[2], 4);
+    memcpy(&out[i].gate_gain, &r[3], 4);
+  }
+  return CRISPY_NS_OK;
+}
+
 int batch_info(const crispy_ns_batch *b, int *streams_per_cta, int *n_ctas, int64_t *launches,
                          int64_t *frames_done) {  // (rnn_streams_per_cta, chunk_frames, ...)
   if (!b) return fail(CRISPY_NS_EINVAL, "batch_info: null handle");
@@ -1546,6 +1632,19 @@ int process_frame(crispy_ns_state *st, float *out480, const float *in480, float 
 int reset(crispy_ns_state *st) {
   if (!st) return fail(CRISPY_NS_EINVAL, "reset: null handle");
   return batch_reset(st->b);
+}
+// the graphs read the controls from the state row, so they need no new capture
+int set_controls(crispy_ns_state *st, const void *c) {
+  if (!st) return fail(CRISPY_NS_EINVAL, "set_controls: null handle");
+  const int id = 0;
+  if (int rc = batch_set_controls(st->b, &id, 1, c, st->s)) return rc;
+  NS_CUDA(cudaStreamSynchronize(st->s));
+  return CRISPY_NS_OK;
+}
+int get_controls(crispy_ns_state *st, void *out) {
+  if (!st) return fail(CRISPY_NS_EINVAL, "get_controls: null handle");
+  const int id = 0;
+  return batch_get_controls(st->b, &id, 1, out);
 }
 
 // ---- a4 / f2: LinearResampler -------------------------------------------------------------------
@@ -2173,6 +2272,55 @@ int multi_reset(crispy_ns_multi *m) {
   for (crispy_ns_batch *b : m->batch) {
     const int rc = batch_reset(b);
     if (rc != CRISPY_NS_OK) return rc;
+  }
+  return CRISPY_NS_OK;
+}
+// global stream ids -> (device block, local ids, entries); checked whole before anything is enqueued
+static int multi_split(const crispy_ns_multi *m, const int *streams, int n, const char *what,
+                       std::vector<std::vector<int>> &local, std::vector<std::vector<int>> &entry) {
+  if (!m) return fail(CRISPY_NS_EINVAL, std::string(what) + ": null handle");
+  if (n < 0 || n > m->n_streams || (n > 0 && !streams))
+    return fail(CRISPY_NS_EINVAL, std::string(what) + ": the stream count must be in [0, n_streams] with a stream list");
+  std::vector<char> seen((size_t)m->n_streams, 0);
+  local.assign(m->batch.size(), {});
+  entry.assign(m->batch.size(), {});
+  for (int i = 0; i < n; i++) {
+    const int s = streams[i];
+    if (s < 0 || s >= m->n_streams) return fail(CRISPY_NS_EINVAL, std::string(what) + ": stream id out of range");
+    if (seen[(size_t)s]) return fail(CRISPY_NS_EINVAL, std::string(what) + ": stream listed twice");
+    seen[(size_t)s] = 1;
+    for (size_t d = 0; d < m->batch.size(); d++)
+      if (s >= m->first[d] && s < m->first[d] + m->count[d]) {
+        local[d].push_back(s - m->first[d]);
+        entry[d].push_back(i);
+      }
+  }
+  return CRISPY_NS_OK;
+}
+int multi_set_controls(crispy_ns_multi *m, const int *streams, int n, const void *controls_v) {
+  const crispy_ns_controls *controls = static_cast<const crispy_ns_controls *>(controls_v);
+  std::vector<std::vector<int>> local, entry;
+  if (int rc = multi_split(m, streams, n, "multi_set_controls", local, entry)) return rc;
+  if (int rc = check_controls(controls, n, "multi_set_controls")) return rc;
+  for (size_t d = 0; d < m->batch.size(); d++) {
+    if (local[d].empty()) continue;
+    std::vector<crispy_ns_controls> c;
+    for (int i : entry[d]) c.push_back(controls[i]);
+    if (int rc = batch_set_controls(m->batch[d], local[d].data(), (int)local[d].size(), c.data(), nullptr)) return rc;
+    NS_CUDA(cudaStreamSynchronize(m->batch[d]->s_k[kNumKernels - 1]));
+  }
+  return CRISPY_NS_OK;
+}
+int multi_get_controls(crispy_ns_multi *m, const int *streams, int n, void *out_v) {
+  crispy_ns_controls *out = static_cast<crispy_ns_controls *>(out_v);
+  std::vector<std::vector<int>> local, entry;
+  if (int rc = multi_split(m, streams, n, "multi_get_controls", local, entry)) return rc;
+  if (n > 0 && !out) return fail(CRISPY_NS_EINVAL, "multi_get_controls: out is null");
+  for (size_t d = 0; d < m->batch.size(); d++) {
+    if (local[d].empty()) continue;
+    std::vector<crispy_ns_controls> c(local[d].size());
+    if (int rc = batch_get_controls(m->batch[d], local[d].data(), (int)local[d].size(), c.data())) return rc;
+    for (size_t j = 0; j < c.size(); j++) out[entry[d][j]] = c[j];
   }
   return CRISPY_NS_OK;
 }

@@ -36,7 +36,7 @@ constexpr int kTabWords = 48;
 //   word 0      : T0 | n_k << 16      (n_k = candidates present, k = 1..n_k)
 //   word 1      : unused
 //   word 2+3(k-1): T_k | pitch_index_k << 16 ; g_k (f32 bits) ; pitch_gain_k (f32 bits)
-constexpr int kRecFloats = 144;
+constexpr int kRecFloats = 148;      // a multiple of 4: K5 stages the record with 16-byte bulk copies
 constexpr int kRecPitchIndex = 0;    // int bits
 constexpr int kRecSilence = 1;       // int bits
 constexpr int kRecPitchGain = 2;
@@ -44,11 +44,13 @@ constexpr int kRecVad = 3;
 constexpr int kRecExp = 4;           // 22 (normalised band correlation)
 constexpr int kRecCeps = 26;         // 22 (DCT of log band energy, offsets applied)
 constexpr int kRecTail = 48;         // 7: features[34..40]
+constexpr int kRecGatePrev = 55;     // the voice gate's output gain G of the previous frame (K4 -> K5)
 constexpr int kRecGRaw = 56;         // 22: band gains as the RNN emits them (the pitch filter uses these)
 constexpr int kRecG = 78;            // 22: band gains after the 0.6*lastg smoothing
 constexpr int kRecEx = 100;          // 22: band energy of the frame
 constexpr int kRecEp = 122;          // 22: band energy of the pitch-lagged window
-static_assert(kRecEp + kBands <= kRecFloats, "record overflow");
+constexpr int kRecGate = 144;        // the voice gate's output gain G of this frame (K4 -> K5)
+static_assert(kRecGate + 1 <= kRecFloats && kRecFloats % 4 == 0, "record overflow");
 constexpr int kSpecStride = 482;     // complex bins per stored spectrum (481 used); per frame: X then P
 
 struct alignas(8) cf {
@@ -73,8 +75,17 @@ constexpr int kStLastGain = kStHp + 2;            // 1
 constexpr int kStLastPeriod = kStLastGain + 1;    // 1 (int bits)
 constexpr int kStMemId = kStLastPeriod + 1;       // 1 (int bits)
 constexpr int kStFrameCount = kStMemId + 1;       // 1 (int bits, informational)
+// per-stream suppression controls (crispy_ns_controls) and the voice gate's carry.  Every field is encoded so that a
+// zeroed row -- a fresh, reset or pre-controls stream -- means no floor and an open gate.
+constexpr int kStCtlMinGain = kStFrameCount + 1;  // 1   : floor on the applied band gains; 0 = none
+constexpr int kStCtlGateThr = kStCtlMinGain + 1;  // 1   : VAD threshold; 0 = every frame voiced = gate off
+constexpr int kStCtlGateHold = kStCtlGateThr + 1; // 1   : frames the gate stays open after a voiced frame (int bits)
+constexpr int kStCtlGateGain = kStCtlGateHold + 1;// 1   : output gain while closed (moot while the threshold is 0)
+constexpr int kStGateLeft = kStCtlGateGain + 1;   // 1   : hold frames left (int bits)
+constexpr int kStGateShut = kStGateLeft + 1;      // 1   : 1 if the previous frame's G was a closed gate's (int bits)
+constexpr int kStGateShutGain = kStGateShut + 1;  // 1   : that G (the gate gain in force then)
 constexpr int kStateFloats = 2784;                // padded to a multiple of 32 floats
-static_assert(kStFrameCount + 1 <= kStateFloats, "state layout overflow");
+static_assert(kStGateShutGain + 1 <= kStateFloats, "state layout overflow");
 
 // ---- per-frame debug taps (optional), mirrors oracle rno_debug
 constexpr int kDbgFeatures = 0;

@@ -2335,6 +2335,39 @@ NS_DEV void features_body(const Params &p, FeatSmem &sm) {
   if (lane == 0) reinterpret_cast<int *>(st)[kStMemId] = memid;
 }
 
+// Voice gate (crispy_ns_controls): a frame is voiced if its returned VAD >= threshold; a voiced frame opens the gate
+// for `hold` more frames; G = 1 while open, else the gate gain.  Serial in time per stream, so both recurrent cores
+// run it where they write the VAD and hand G of the frame and of the one before to K5 in the record (K5's runs of a
+// chunk are concurrent and could not carry it).  A zeroed state row is threshold 0: every frame voiced, G = 1.
+struct GateState {
+  float thr, gain, shut_gain;
+  int hold, left, shut;
+};
+NS_DEV GateState gate_load(const float *st) {
+  const int *sti = reinterpret_cast<const int *>(st);
+  return GateState{st[kStCtlGateThr], st[kStCtlGateGain], st[kStGateShutGain], sti[kStCtlGateHold], sti[kStGateLeft],
+                   sti[kStGateShut]};
+}
+NS_DEV void gate_step(GateState &q, float vad, float *rec) {
+  bool open = true;
+  if (!(vad < q.thr))  // vad >= thr; a NaN VAD (non-finite input) counts as voiced, so an unset gate never closes
+    q.left = q.hold;
+  else if (q.left > 0)
+    q.left -= 1;
+  else
+    open = false;
+  rec[kRecGatePrev] = q.shut ? q.shut_gain : 1.f;
+  rec[kRecGate] = open ? 1.f : q.gain;
+  q.shut = open ? 0 : 1;
+  q.shut_gain = open ? 0.f : q.gain;
+}
+NS_DEV void gate_save(const GateState &q, float *st) {
+  int *sti = reinterpret_cast<int *>(st);
+  sti[kStGateLeft] = q.left;
+  sti[kStGateShut] = q.shut;
+  st[kStGateShutGain] = q.shut_gain;
+}
+
 // =================================================================================================
 // K4: a14 the recurrent core on the tensor pipe, 16 streams per CTA, serial over the chunk's frames.
 // All weights stay in shared memory as bf16 B fragments for the whole launch; every activation
@@ -2470,6 +2503,12 @@ NS_DEV void rnn_body(const Params &p, RnnSmem &r) {
   load4(hd[0], kStHDen, warp * 8 + c2, 96);
   load4(hd[1], kStHDen, (warp + 8) * 8 + c2, warp < 4 ? 96 : 0);
   load4(lastg, kStLastG, warp * 8 + c2, warp < 3 ? kBands : 0);
+  // the voice gate runs on the lanes that write the VAD (warp 7, lane % 4 == 0: streams srow[0], srow[1])
+  const bool gate_lane = warp == 7 && (lane & 3) == 0;
+  GateState gate[2] = {};
+#pragma unroll
+  for (int h = 0; h < 2; h++)
+    if (gate_lane && live[h]) gate[h] = gate_load(p.state + (long long)srow[h] * kStateFloats);
   Simt::cta_sync();  // the fragments were cleared
   if (warp < 3) store_frag(r, kPosVadH + warp * 8, lane, hv);
   if (warp < 6) store_frag(r, kPosNoiseH + warp * 8, lane, hn);
@@ -2631,12 +2670,14 @@ NS_DEV void rnn_body(const Params &p, RnnSmem &r) {
           *reinterpret_cast<cf *>(rec + kRecG + band) = cf{gout[2 * h], gout[2 * h + 1]};
         }
       }
-    } else if (warp == 7 && (lane & 3) == 0) {
+    } else if (gate_lane) {
 #pragma unroll
       for (int h = 0; h < 2; h++) {
         if (live[h]) {
           const float v = sil[h] ? 0.f : vad[h];
-          p.rec[((long long)srow[h] * p.chunk_cap + t) * kRecFloats + kRecVad] = v;
+          float *rec = p.rec + ((long long)srow[h] * p.chunk_cap + t) * kRecFloats;
+          rec[kRecVad] = v;
+          gate_step(gate[h], v, rec);
           if (p.vad) p.vad[(long long)srow[h] * p.vad_stride + p.frame0 + t] = v;
         }
       }
@@ -2649,13 +2690,17 @@ NS_DEV void rnn_body(const Params &p, RnnSmem &r) {
   save4(hd[0], kStHDen, warp * 8 + c2, 96);
   save4(hd[1], kStHDen, (warp + 8) * 8 + c2, warp < 4 ? 96 : 0);
   save4(lastg, kStLastG, warp * 8 + c2, warp < 3 ? kBands : 0);
+#pragma unroll
+  for (int h = 0; h < 2; h++)
+    if (gate_lane && live[h]) gate_save(gate[h], p.state + (long long)srow[h] * kStateFloats);
 }
 
 // =================================================================================================
 // K5: a15 pitch filter + gain interpolation, a16 synthesis; one 128-thread group per stream walks
 // the chunk's frames carrying synthesis_mem in shared memory
 // =================================================================================================
-NS_DEV void pitch_filter_and_gains(const Grp &g, const Tab &T, SpecSmem &s, cf *X, const cf *P, const float *rc) {
+// min_gain (crispy_ns_controls): floor on the applied band gains; lastg and the pitch filter keep the unfloored ones
+NS_DEV void pitch_filter_and_gains(const Grp &g, const Tab &T, SpecSmem &s, cf *X, const cf *P, const float *rc, float min_gain) {
   if (g.tid < kBands) {
     const int i = g.tid;
     const float e = rc[kRecExp + i], gi = rc[kRecGRaw + i];
@@ -2715,7 +2760,12 @@ NS_DEV void pitch_filter_and_gains(const Grp &g, const Tab &T, SpecSmem &s, cf *
     const int k0 = 4 * g.tid, b = T.bin_band(k0);
     const f4 fr4 = T.bin_frac4(k0);
     const float fr[4] = {fr4.x, fr4.y, fr4.z, fr4.w};
-    const float n0 = s.nrm[b], n1 = s.nrm[b + 1], g0 = rc[kRecG + b], g1 = rc[kRecG + b + 1];
+    const float n0 = s.nrm[b], n1 = s.nrm[b + 1];
+    float g0 = rc[kRecG + b], g1 = rc[kRecG + b + 1];
+    if (min_gain > 0.f) {  // uniform per stream: the default path skips it
+      g0 = fmaxf(g0, min_gain);
+      g1 = fmaxf(g1, min_gain);
+    }
     const bool sw = (g.tid & 4) != 0;
     f4 xq[2];
     ld_slot(X + k0, sw, xq[0], xq[1]);
@@ -2754,7 +2804,8 @@ NS_DEV int16_t out_mix(const Params &p, float o, float app) {
 }
 NS_DEV uint32_t pack16(int16_t lo, int16_t hi) { return (uint32_t)(uint16_t)lo | ((uint32_t)(uint16_t)hi << 16); }
 
-NS_DEV void store_frame(const Grp &g, const Tab &T, const Params &p, SpecSmem &s, const cf *X, int stream, int t_call) {
+NS_DEV void store_frame(const Grp &g, const Tab &T, const Params &p, SpecSmem &s, const cf *X, const float *rc, int stream,
+                        int t_call) {
   // X holds z[m] with x[2m] = z.x, x[2m+1] = -z.y.  out[i] = x[i] w[i] + synth[i]; synth = x[480+i] w[479-i]
   const int slot = t_call + p.out_frame_offset;
   const float *zb = reinterpret_cast<const float *>(X);
@@ -2762,9 +2813,14 @@ NS_DEV void store_frame(const Grp &g, const Tab &T, const Params &p, SpecSmem &s
   const int i = 4 * g.tid;
   const f4 za = ld4(zb + i), zc = ld4(zb + kFrame + i), wa = T.win4(i), wr = T.win4(kFrame - 4 - i);
   const f4 sy = ld4(s.synth + i);
-  const float o[4] = {za.x * wa.x + sy.x, (-za.y) * wa.y + sy.y, za.z * wa.z + sy.z, (-za.w) * wa.w + sy.w};
+  float o[4] = {za.x * wa.x + sy.x, (-za.y) * wa.y + sy.y, za.z * wa.z + sy.z, (-za.w) * wa.w + sy.w};
   *reinterpret_cast<f4 *>(s.synth + i) = f4{zc.x * wr.w, (-zc.y) * wr.z, zc.z * wr.y, (-zc.w) * wr.x};
   if (slot < 0) return;
+  const float gp = rc[kRecGatePrev], gc = rc[kRecGate];
+  if (gp != 1.f || gc != 1.f) {  // the voice gate's ramp from G of the previous frame to G of this one; uniform per frame
+#pragma unroll
+    for (int u = 0; u < 4; u++) o[u] = o[u] * (gp + (gc - gp) * ((float)(i + u + 1) / 480.0f));
+  }
   const long long o_off = (long long)stream * p.out_stride + (long long)slot * kFrame + i;
   const bool vec_out = ((reinterpret_cast<uintptr_t>(p.out) & 15) == 0) && ((p.out_stride & 3) == 0);
   if (p.flags & kFlagMixStereoI16) {
@@ -2829,7 +2885,7 @@ inline int pick_syn_run(int n_streams, int n_frames, int resident_ctas) {
   return best;
 }
 
-// one thread stages a frame's spectra (X | P, 7,712 B) and record (576 B) into buffer b: two bulk copies on s.mbar
+// one thread stages a frame's spectra (X | P, 7,712 B) and record (592 B) into buffer b: two bulk copies on s.mbar
 NS_DEV void synth_stage(const Grp &g, const Params &p, SpecSmem &s, int stream, int t, int b) {
   static_assert((2 * kSpecStride * sizeof(cf)) % 16 == 0 && (kRecFloats * sizeof(float)) % 16 == 0, "bulk copy sizes");
   if (g.tid == 0) {
@@ -2841,11 +2897,12 @@ NS_DEV void synth_stage(const Grp &g, const Params &p, SpecSmem &s, int stream, 
   }
 }
 
-NS_DEV void synth_frame(const Grp &g, const Tab &T, const Params &p, SpecSmem &s, int stream, int t, bool halo, int b) {
+NS_DEV void synth_frame(const Grp &g, const Tab &T, const Params &p, SpecSmem &s, int stream, int t, bool halo, int b,
+                        float min_gain) {
   cf *X = s.spec[b], *P = X + kSpecStride;
   const float *rc = s.rec_s[b];
   const bool silent = reinterpret_cast<const int *>(rc)[kRecSilence] != 0;
-  if (!silent) pitch_filter_and_gains(g, T, s, X, P, rc);
+  if (!silent) pitch_filter_and_gains(g, T, s, X, P, rc, min_gain);
   if (p.dbg && !halo) {
     float *d = p.dbg + ((long long)stream * p.n_frames_call + p.frame0 + t) * kDbgFloats;
     if (g.tid < kBands) d[kDbgGains + g.tid] = rc[kRecG + g.tid];
@@ -2865,7 +2922,7 @@ NS_DEV void synth_frame(const Grp &g, const Tab &T, const Params &p, SpecSmem &s
       s.synth[i] = x1 * T.win(kFrame - 1 - i);
     }
   } else {
-    store_frame(g, T, p, s, X, stream, p.frame0 + t);
+    store_frame(g, T, p, s, X, rc, stream, p.frame0 + t);
   }
   gsync(g);
 }
@@ -2888,6 +2945,7 @@ NS_DEV void synthesis_body(const Params &p, SpecSmem &s) {
     const int stream = task / runs, t0 = (task - stream * runs) * run;
     const int t1 = (t0 + run < p.n_frames) ? t0 + run : p.n_frames;
     float *st = p.state + (long long)stream * kStateFloats;
+    const float min_gain = st[kStCtlMinGain];  // set between calls only: no kernel of this call writes it
     // a run that does not start the chunk re-synthesises the frame before it (the overlap-add halo)
     const int first = (t0 == 0) ? 0 : t0 - 1;
     synth_stage(g, p, s, stream, first, 0);
@@ -2899,7 +2957,7 @@ NS_DEV void synthesis_body(const Params &p, SpecSmem &s) {
       parity ^= 1u;
       gsync(g);  // frame t has landed in buffer b; everyone is done with buffer b ^ 1
       if (t + 1 < t1) synth_stage(g, p, s, stream, t + 1, b ^ 1);  // in flight while frame t is worked on
-      synth_frame(g, T, p, s, stream, t, t < t0, b);
+      synth_frame(g, T, p, s, stream, t, t < t0, b, min_gain);
     }
     if (t1 == p.n_frames) {
       for (int i = g.tid; i < kFrame; i += kGroupThreads) st[kStSynth + (1 - p.synth_sel) * kFrame + i] = s.synth[i];

@@ -214,6 +214,9 @@ __device__ __forceinline__ void rnn_tc5_body(const Params &p, Smem &s) {
 #pragma unroll
     for (int j = 0; j < 6; j++) lastg[j] = (live && 6 * hs + j < kBands) ? st[kStLastG + 6 * hs + j] : 0.f;
   }
+  // the voice gate (ns_pipe.cuh gate_step) runs on the thread that writes the stream's VAD
+  GateState gate = {};
+  if (live && hs == 0) gate = gate_load(p.state + (long long)stream * kStateFloats);
   store_act<6, 1>(lane_base, kPosVadH + 6 * hs, hv);
   store_act<12, 2>(lane_base, kPosNoiseH + 12 * hs, hn);
   store_act<24, 4>(lane_base, kPosDenH + 24 * hs, hd);
@@ -438,6 +441,7 @@ __device__ __forceinline__ void rnn_tc5_body(const Params &p, Smem &s) {
       if (hs == 0) {
         const float v = sil ? 0.f : vad;
         rec[kRecVad] = v;
+        gate_step(gate, v, rec);
         if (p.vad) p.vad[(long long)stream * p.vad_stride + p.frame0 + t] = v;
       }
     }
@@ -454,6 +458,7 @@ __device__ __forceinline__ void rnn_tc5_body(const Params &p, Smem &s) {
 #pragma unroll
     for (int j = 0; j < 6; j++)
       if (6 * hs + j < kBands) st[kStLastG + 6 * hs + j] = lastg[j];
+    if (hs == 0) gate_save(gate, st);
     if (err && tid == 0) reinterpret_cast<int *>(st)[kStFrameCount] = -1;  // poison the informational frame counter
   }
 #ifdef NS_TC5_CLOCKS

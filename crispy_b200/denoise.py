@@ -76,6 +76,35 @@ class Model:
             pass
 
 
+def _controls(n, min_gain, atten_limit_db, vad_threshold, hold_frames, gate_gain):
+    """n crispy_ns_controls; every argument is a scalar or one value per stream.  The library checks the ranges."""
+    if min_gain is not None and atten_limit_db is not None:
+        raise CrispyNsError("give min_gain or atten_limit_db, not both")
+    if atten_limit_db is not None:
+        min_gain = np.power(10.0, -np.asarray(atten_limit_db, dtype=np.float64) / 20.0)
+    cols = [np.broadcast_to(np.asarray(v, dtype=dt), (n,)) for v, dt in
+            ((0.0 if min_gain is None else min_gain, np.float32), (vad_threshold, np.float32),
+             (hold_frames, np.int64), (gate_gain, np.float32))]
+    arr = (_lib.Controls * max(n, 1))()
+    for i in range(n):
+        h = int(cols[2][i])
+        arr[i] = _lib.Controls(float(cols[0][i]), float(cols[1][i]), h if -2**31 <= h < 2**31 else -1, float(cols[3][i]))
+    return arr
+
+
+def _controls_dicts(arr, n):
+    return [{"min_gain": arr[i].min_gain, "vad_threshold": arr[i].gate_threshold, "hold_frames": arr[i].gate_hold,
+             "gate_gain": arr[i].gate_gain} for i in range(n)]
+
+
+_CONTROLS_DOC = """Per-stream suppression controls (include/crispy_ns.h crispy_ns_controls), taking effect from the stream's next
+        frame.  min_gain (or atten_limit_db, min_gain = 10^(-dB/20)) floors every band gain applied to the spectrum;
+        None / 0 is no limit.  The voice gate mutes (gate_gain 0) or attenuates the output of frames whose VAD stays
+        below vad_threshold for more than hold_frames frames after the last voiced one, with a linear ramp over each
+        frame; vad_threshold 0 turns it off.  A value out of range raises CrispyNsError and changes nothing.  The controls
+        belong to the recording in the slot: every reset turns them off, and stream records carry them."""
+
+
 class DenoiseState:
     """Mirror of nnnoiseless::DenoiseState as the reference uses it (audio.rs:203, :229, :268)."""
 
@@ -104,6 +133,18 @@ class DenoiseState:
 
     def reset(self) -> None:
         check(_lib.lib().crispy_ns_reset(self._h))
+
+    def set_controls(self, *, min_gain=None, atten_limit_db=None, vad_threshold=0.0, hold_frames=0,
+                     gate_gain=0.0) -> None:
+        c = _controls(1, min_gain, atten_limit_db, vad_threshold, hold_frames, gate_gain)
+        check(_lib.lib().crispy_ns_set_controls(self._h, c))
+
+    def get_controls(self) -> dict:
+        c = _lib.Controls()
+        check(_lib.lib().crispy_ns_get_controls(self._h, C.byref(c)))
+        return _controls_dicts([c], 1)[0]
+
+    set_controls.__doc__ = _CONTROLS_DOC
 
     def __del__(self):
         try:
@@ -475,6 +516,23 @@ class BatchDenoiser:
         st = torch.cuda.current_stream(self.device).cuda_stream
         check(_lib.lib().crispy_ns_batch_reset_streams(self._h, ptr, int(ids.size), st))
 
+    def set_controls(self, streams, *, min_gain=None, atten_limit_db=None, vad_threshold=0.0, hold_frames=0,
+                     gate_gain=0.0) -> None:
+        import torch
+        ids, ptr = self._ids(streams)
+        c = _controls(int(ids.size), min_gain, atten_limit_db, vad_threshold, hold_frames, gate_gain)
+        st = torch.cuda.current_stream(self.device).cuda_stream
+        check(_lib.lib().crispy_ns_batch_set_controls(self._h, ptr, int(ids.size), c, st))
+
+    set_controls.__doc__ = _CONTROLS_DOC + """  Ordered on the current torch CUDA stream as reset_streams."""
+
+    def get_controls(self, streams) -> list:
+        """[{min_gain, vad_threshold, hold_frames, gate_gain}] of the listed streams (synchronous)."""
+        ids, ptr = self._ids(streams)
+        c = (_lib.Controls * max(int(ids.size), 1))()
+        check(_lib.lib().crispy_ns_batch_get_controls(self._h, ptr, int(ids.size), c))
+        return _controls_dicts(c, int(ids.size))
+
     def save_streams(self, streams) -> bytes:
         """One self-describing record per listed stream (stream_state_size() bytes each), concatenated."""
         ids, ptr = self._ids(streams)
@@ -568,6 +626,27 @@ class MultiDenoiser:
 
     def reset(self) -> None:
         check(_lib.lib().crispy_ns_multi_reset(self._h))
+
+    def _ids(self, streams):
+        ids = np.ascontiguousarray(np.asarray(streams, dtype=np.int64).reshape(-1))
+        if ids.size and (ids.min() < 0 or ids.max() >= self.n_streams):
+            raise CrispyNsError("stream id out of range")
+        ids = ids.astype(np.int32)
+        return ids, ids.ctypes.data_as(C.POINTER(C.c_int))
+
+    def set_controls(self, streams, *, min_gain=None, atten_limit_db=None, vad_threshold=0.0, hold_frames=0,
+                     gate_gain=0.0) -> None:
+        ids, ptr = self._ids(streams)
+        c = _controls(int(ids.size), min_gain, atten_limit_db, vad_threshold, hold_frames, gate_gain)
+        check(_lib.lib().crispy_ns_multi_set_controls(self._h, ptr, int(ids.size), c))
+
+    set_controls.__doc__ = _CONTROLS_DOC + """  streams are the handle's global ids; synchronous."""
+
+    def get_controls(self, streams) -> list:
+        ids, ptr = self._ids(streams)
+        c = (_lib.Controls * max(int(ids.size), 1))()
+        check(_lib.lib().crispy_ns_multi_get_controls(self._h, ptr, int(ids.size), c))
+        return _controls_dicts(c, int(ids.size))
 
     def process_streams_host(self, x, *, unit_scale: bool = True, volume: float = 1.0, drop_first_frame: bool = False,
                              out=None, vad=None, out_i16: bool = False, app=None, mix_stereo_i16: bool = False,

@@ -187,6 +187,43 @@ size_t crispy_ns_stream_state_size(void);
 int crispy_ns_batch_save_streams(crispy_ns_batch *b, const int *streams, int n, void *buf, size_t len);
 int crispy_ns_batch_load_streams(crispy_ns_batch *b, const int *streams, int n, const void *buf, size_t len);
 
+/* ---- per-stream suppression controls: an attenuation limit and a voice gate.  They act only on what leaves the
+ * pipeline: no pitch decision, VAD or recurrent state depends on them.
+ *   Attenuation limit: on non-silent frames the band gains applied to the spectrum are max(g, min_gain), where
+ *     g = max(g_raw, 0.6 lastg) is the smoothed gain; lastg keeps the unfloored g and the pitch filter uses g_raw.
+ *     Silent frames pass through as without it.  The floor changes synthesis_mem.
+ *   Voice gate: frame t is voiced if its returned VAD (0 on silent frames) >= gate_threshold.  A voiced frame sets
+ *     left = gate_hold and the gate is open; otherwise, if left > 0, left -= 1 and the gate is open; otherwise it is
+ *     closed.  G_t = 1 while open, else gate_gain.  Output sample i of frame t is the 16-bit-scale denoised sample
+ *     times G_{t-1} + (G_t - G_{t-1}) * ((float)(i + 1) / 480.0f), every operation rounded separately, taken after
+ *     the overlap-add and before the output conversion (unit scale, clamp, volume, i16, and the dual-mono mix, whose
+ *     app audio is not gated).  The gate never writes synthesis_mem; CRISPY_NS_DROP_FIRST_FRAME drops a gated frame
+ *     and the gate still advances.  A fresh stream has G_{-1} = 1.
+ *   All zeros (a fresh stream) is no floor and the gate off; gate_gain matters only while gate_threshold > 0.
+ * The controls and the gate's carry (left, G of the last frame) belong to the recording in the slot: they are part of
+ * the stream's state, so subset calls, stream records and whole-batch states carry them, records saved before the
+ * controls existed load with them off, and every reset (crispy_ns_reset, _batch_reset, _reset_async, _reset_streams)
+ * turns them off.  Setting the controls keeps the gate's carry: they take effect from the stream's next frame.
+ * set_controls is ordered as crispy_ns_batch_reset_streams: after every call already enqueued and before the next one,
+ * whichever CUDA stream that call is made on; cuda_stream waits for it.  get_controls is synchronous.  A value out of
+ * range or NaN, a null handle or array, or a stream id out of range or listed twice gives CRISPY_NS_EINVAL and changes
+ * no state. ---- */
+typedef struct {
+  float min_gain;        /* [0, 1]; floor on every band gain applied to the spectrum; 0 = no limit (today) */
+  float gate_threshold;  /* [0, 1]; a frame is voiced if its VAD >= threshold; 0 = every frame voiced = gate off */
+  int32_t gate_hold;     /* [0, 1<<20] frames the gate stays open after the last voiced frame */
+  float gate_gain;       /* [0, 1]; output gain while the gate is closed; 0 = mute */
+} crispy_ns_controls;
+/* controls / out point to n crispy_ns_controls structs, one for the single-stream calls.  The prototypes spell them as void
+ * pointers because every prototype of this header uses only scalar, handle and void pointer types, which the Rust
+ * shim's extern block (bindings/rust/ns_gpu.rs) is checked against type by type; the shim's methods take the
+ * #[repr(C)] struct. */
+int crispy_ns_batch_set_controls(crispy_ns_batch *b, const int *streams, int n, const void *controls, void *cuda_stream);
+int crispy_ns_batch_get_controls(crispy_ns_batch *b, const int *streams, int n, void *out);
+/* the same for the one stream of a crispy_ns_state handle, synchronously */
+int crispy_ns_set_controls(crispy_ns_state *st, const void *controls);
+int crispy_ns_get_controls(crispy_ns_state *st, void *out);
+
 /* launch geometry + bookkeeping: streams per recurrent-core CTA, frames per engine chunk
  * ($CRISPY_NS_CHUNK_FRAMES overrides the default at batch_create), kernels launched so far,
  * frames processed per stream */
@@ -217,6 +254,9 @@ int crispy_ns_multi_reset(crispy_ns_multi *m);
 int crispy_ns_multi_process_streams_host(crispy_ns_multi *m, const void *h_in, void *h_out, float *h_vad,
                                          const float *h_app, int n_frames, int64_t in_stride, int64_t out_stride,
                                          int64_t vad_stride, int64_t app_stride, uint32_t flags, float volume);
+/* crispy_ns_batch_set_controls / _get_controls over the multi handle's global stream ids (synchronous) */
+int crispy_ns_multi_set_controls(crispy_ns_multi *m, const int *streams, int n, const void *controls);
+int crispy_ns_multi_get_controls(crispy_ns_multi *m, const int *streams, int n, void *out);
 void crispy_ns_multi_destroy(crispy_ns_multi *m);
 
 /* pinned host memory for the host-pointer path */

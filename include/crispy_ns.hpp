@@ -88,6 +88,10 @@ inline std::size_t f32_as_usize(float v) {
 
 inline int device_count() { return crispy_ns_device_count(); }
 
+// Per-stream suppression controls (crispy_ns_controls): a floor on the applied band gains and a voice gate with hold.
+// Value-initialised, they are off.  The setters throw crispy::Error for a value out of range or NaN.
+using Controls = crispy_ns_controls;
+
 // The six int8 layers of the recurrent network.  nnnoiseless embeds its weights in the crate; here they are data
 // (crispy_ns_model_*): a CRNSMDL1 / rnnoise-nu blob, or seeded synthetic weights of the same topology.
 class Model {
@@ -156,6 +160,12 @@ class DenoiseState {
     return process_frame(output.data(), output.size(), input.data(), input.size());
   }
   void reset() { detail::check(crispy_ns_reset(h_)); }  // a fresh state, as the model switch at audio.rs:955-965 builds
+  void set_controls(const Controls &c) { detail::check(crispy_ns_set_controls(h_, &c)); }
+  Controls controls() {
+    Controls c{};
+    detail::check(crispy_ns_get_controls(h_, &c));
+    return c;
+  }
   DenoiseState(const DenoiseState &) = delete;
   DenoiseState &operator=(const DenoiseState &) = delete;
   ~DenoiseState() { crispy_ns_destroy(h_); }
@@ -358,6 +368,16 @@ class BatchDenoiser {
   void load_streams(const std::vector<int> &streams, const std::vector<std::uint8_t> &b) {
     detail::check(crispy_ns_batch_load_streams(h_, streams.data(), (int)streams.size(), b.data(), b.size()));
   }
+  // controls[i] for streams[i]; ordered as reset_streams
+  void set_controls(const std::vector<int> &streams, const std::vector<Controls> &controls, void *cuda_stream = nullptr) {
+    if (controls.size() != streams.size()) throw Error(CRISPY_NS_EINVAL, "set_controls: one Controls per stream");
+    detail::check(crispy_ns_batch_set_controls(h_, streams.data(), (int)streams.size(), controls.data(), cuda_stream));
+  }
+  std::vector<Controls> controls(const std::vector<int> &streams) {
+    std::vector<Controls> c(streams.size());
+    detail::check(crispy_ns_batch_get_controls(h_, streams.data(), (int)streams.size(), c.data()));
+    return c;
+  }
   crispy_ns_batch *get() { return h_; }
 
  private:
@@ -395,6 +415,16 @@ class MultiDenoiser {
                                                        CRISPY_NS_IN_I16 | CRISPY_NS_OUT_I16, 1.0f));
   }
   void reset() { detail::check(crispy_ns_multi_reset(h_)); }
+  // global stream ids; synchronous
+  void set_controls(const std::vector<int> &streams, const std::vector<Controls> &controls) {
+    if (controls.size() != streams.size()) throw Error(CRISPY_NS_EINVAL, "set_controls: one Controls per stream");
+    detail::check(crispy_ns_multi_set_controls(h_, streams.data(), (int)streams.size(), controls.data()));
+  }
+  std::vector<Controls> controls(const std::vector<int> &streams) {
+    std::vector<Controls> c(streams.size());
+    detail::check(crispy_ns_multi_get_controls(h_, streams.data(), (int)streams.size(), c.data()));
+    return c;
+  }
 
  private:
   crispy_ns_multi *h_ = nullptr;
