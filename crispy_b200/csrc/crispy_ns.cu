@@ -77,24 +77,13 @@ __global__ void __launch_bounds__(kPitchThreads) ns_pitch_kernel(const __grid_co
   ns::pitch_body7<kPitchRun, kPitchThreads>(p, *reinterpret_cast<PitchShared *>(smem_raw));
 #endif
 }
-#ifndef NS_PITCH_V7
-constexpr int kPitchPolicies = 3;
-#else
-constexpr int kPitchPolicies = 1;
-#endif
+static_assert(ns::kSumMask == CRISPY_NS_SUM_MASK && ns::kBiquadF32 == CRISPY_NS_BIQUAD_F32, "numerics bits");
 typedef void (*KernelFn)(ns::Params);
 static KernelFn pitch_kernel(uint32_t numerics) {
-#ifndef NS_PITCH_V7
-  switch (numerics & CRISPY_NS_SUM_MASK) {
-    case CRISPY_NS_SUM_DOT4: return ns_pitch_kernel<1>;
-    case CRISPY_NS_SUM_DOT4_XCORR: return ns_pitch_kernel<2>;
-    default: break;
-  }
-#endif
-  return ns_pitch_kernel<0>;
+  return ns::with_sum_order(numerics, [](auto sp) -> KernelFn { return ns_pitch_kernel<decltype(sp)::value>; });
 }
 static KernelFn highpass_kernel(uint32_t numerics) {
-  return (numerics & CRISPY_NS_BIQUAD_F32) ? ns_highpass_kernel<true> : ns_highpass_kernel<false>;
+  return ns::biquad_f32(numerics) ? ns_highpass_kernel<true> : ns_highpass_kernel<false>;
 }
 __global__ void __launch_bounds__(32 * kScanWarps) ns_pitchscan_kernel(const __grid_constant__ ns::Params p) {
   ns::pitchscan_body(p, kScanWarps);
@@ -591,7 +580,7 @@ static cudaError_t configure_kernels(int dev) {
     e = cudaFuncSetAttribute(ns_highpass_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kHpExclusiveSmem);
   if (e == cudaSuccess)
     e = cudaFuncSetAttribute(ns_highpass_par_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kHpExclusiveSmem);
-  for (int sp = 0; sp < kPitchPolicies && e == cudaSuccess; sp++)
+  for (int sp = 0; sp < ns::kSumOrders && e == cudaSuccess; sp++)
     e = cudaFuncSetAttribute(pitch_kernel((uint32_t)sp), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(PitchShared));
   if (e == cudaSuccess)
     e = cudaFuncSetAttribute(ns_spectrum_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(ns::SpecSmem));
@@ -606,13 +595,12 @@ static cudaError_t configure_kernels(int dev) {
 }
 
 // K0's form for a call over n streams ($CRISPY_NS_HP_EXCLUSIVE / $CRISPY_NS_HP_PAR as read at batch_create win).  Both
-// forms give the same bits, so a subset call may pick the form for its own size.  The parallel form speculates the f64
-// expression only: under CRISPY_NS_BIQUAD_F32 the single recursion warp runs (its f32 chain is a few dependent f32
-// operations a sample instead of the f64 chain's 74 cycles).
+// forms give the same bits, so a subset call may pick the form for its own size.  Under CRISPY_NS_BIQUAD_F32 the single
+// recursion warp runs (ns::hp_par_form; its f32 chain is a few dependent f32 operations a sample instead of the f64
+// chain's 74 cycles).
 static void pick_hp_form(const crispy_ns_batch *b, int n, bool *exclusive, bool *par) {
   *exclusive = b->hp_exclusive_env >= 0 ? b->hp_exclusive_env != 0 : n <= NS_HP_EXCLUSIVE_MAX_STREAMS;
-  *par = b->hp_par_env >= 0 ? b->hp_par_env != 0 : (NS_HP_PAR != 0 && *exclusive);
-  if (b->numerics & CRISPY_NS_BIQUAD_F32) *par = false;
+  *par = ns::hp_par_form(b->numerics, b->hp_par_env >= 0 ? b->hp_par_env != 0 : (NS_HP_PAR != 0 && *exclusive));
 }
 
 static cudaError_t prof_begin(crispy_ns_batch *b, int kernel, cudaStream_t s) {
@@ -714,30 +702,11 @@ static int run_device(crispy_ns_batch *b, const void *d_in, void *d_out, float *
                                   "longer share a first frame (reset or load the whole batch first)");
   NS_CUDA(cudaSetDevice(b->device));
   NS_CUDA(configure_kernels(b->device));
-  ns::Params p;
-  memset(&p, 0, sizeof(p));
-  p.in = d_in;
-  p.out = d_out;
-  p.vad = d_vad;
-  p.app = d_app;
-  p.dbg = d_taps;
-  p.state = n_rows > 0 ? b->d_rows : b->d_state;
-  p.tables = b->d_tables;
-  p.rnn_hdr = b->d_hdr;
-  p.rnn_words = b->d_words;
-  p.rnn_bias = b->d_bias;
-  p.in_stride = in_stride;
-  p.out_stride = out_stride;
-  p.vad_stride = vad_stride;
-  p.app_stride = app_stride;
-  p.hp_stride = ns::kHist + (long long)b->chunk_cap * ns::kFrame;
-  p.n_streams = n_rows > 0 ? n_rows : b->n_streams;
-  p.n_frames_call = n_frames;
-  p.chunk_cap = b->chunk_cap;
-  p.out_frame_offset = ((flags & CRISPY_NS_DROP_FIRST_FRAME) && b->frames_done == 0) ? -1 : 0;
-  p.flags = flags & 0xFFu;
-  p.volume = volume;
-  const int n = p.n_streams;
+  const int n = n_rows > 0 ? n_rows : b->n_streams;
+  ns::Params p = ns::call_params(d_in, d_out, d_vad, d_app, d_taps, n_rows > 0 ? b->d_rows : b->d_state, b->d_tables,
+                                 b->d_hdr, b->d_words, b->d_bias, in_stride, out_stride, vad_stride, app_stride, n, n_frames,
+                                 b->chunk_cap, ((flags & CRISPY_NS_DROP_FIRST_FRAME) && b->frames_done == 0) ? -1 : 0,
+                                 flags & 0xFFu, volume);
   const int groups = (n + ns::kMmaStreams - 1) / ns::kMmaStreams;
   bool hp_par = b->hp_par, hp_exclusive = b->hp_exclusive;
   if (n_rows > 0) pick_hp_form(b, n, &hp_exclusive, &hp_par);
@@ -763,14 +732,8 @@ static int run_device(crispy_ns_batch *b, const void *d_in, void *d_out, float *
   for (int f0 = 0; f0 < n_frames; f0 += b->chunk_cap) {
     const int slot = (int)(b->chunks_done % kSlots);
     const int nf = (n_frames - f0) < b->chunk_cap ? (n_frames - f0) : b->chunk_cap;
-    p.frame0 = f0;
-    p.n_frames = nf;
-    p.hp = b->d_hp[slot];
-    p.tab = b->d_tab[slot];
-    p.rec = b->d_rec[slot];
-    p.spec = b->d_spec[slot];
-    p.featq = b->d_featq[slot];
-    p.synth_sel = (int)(b->chunks_done & 1);
+    ns::set_chunk(p, f0, nf, b->d_hp[slot], b->d_tab[slot], b->d_rec[slot], b->d_spec[slot], b->d_featq[slot],
+                  (int)(b->chunks_done & 1));
     // the slot's previous chunk must have left the pipeline before K0 overwrites its workspace
     if (b->chunks_done >= kSlots) NS_CUDA(cudaStreamWaitEvent(b->s_k[0], b->e_k[slot][kNumKernels - 1], 0));
     for (int k = 0; k < kNumKernels; k++) {
@@ -845,7 +808,7 @@ int model_to_bytes(const crispy_ns_model *m, void *buf, size_t cap, size_t *need
 void model_destroy(crispy_ns_model *m) { delete m; }
 int model_set_numerics(crispy_ns_model *m, uint32_t numerics) {
   if (!m) return fail(CRISPY_NS_EINVAL, "model_set_numerics: model is null");
-  if ((numerics & ~(uint32_t)(CRISPY_NS_SUM_MASK | CRISPY_NS_BIQUAD_F32)) || (numerics & CRISPY_NS_SUM_MASK) == CRISPY_NS_SUM_MASK)
+  if (!ns::numerics_valid(numerics))
     return fail(CRISPY_NS_EINVAL, "model_set_numerics: unknown bits, or sum order 3");
   m->numerics = numerics;
   return CRISPY_NS_OK;
@@ -917,10 +880,8 @@ int batch_create(const crispy_ns_model *model, int device, int n_streams, crispy
   if (ndev == 0) return fail(CRISPY_NS_ENODEV, "no CUDA device: libcrispy_ns has no CPU fallback");
   if (device < 0 || device >= ndev) return fail(CRISPY_NS_ENODEV, "device index out of range");
   const uint32_t numerics = model_numerics(model);
-#ifdef NS_PITCH_V7
-  if (numerics & CRISPY_NS_SUM_MASK)
+  if ((int)(numerics & ns::kSumMask) >= ns::kSumOrders)
     return fail(CRISPY_NS_EINVAL, "batch_create: this build's pitch kernel (NS_PITCH_V7) sums in the sequential order only");
-#endif
   ns::Model local;
   const ns::Model *m = nullptr;
   if (model) {
@@ -1065,6 +1026,21 @@ int process_streams_debug(crispy_ns_batch *b, const void *d_in, void *d_out, flo
                     flags, volume, (cudaStream_t)cuda_stream);
 }
 
+// grows the pair of device buffers d to `bytes` each when their capacity cap is smaller
+template <class T>
+static cudaError_t fit_pair(T *(&d)[2], size_t &cap, size_t bytes) {
+  if (cap >= bytes) return cudaSuccess;
+  for (int i = 0; i < 2; i++) {
+    cudaFree(d[i]);
+    d[i] = nullptr;
+  }
+  cap = 0;
+  for (int i = 0; i < 2; i++)
+    if (cudaError_t e = cudaMalloc((void **)&d[i], bytes); e != cudaSuccess) return e;
+  cap = bytes;
+  return cudaSuccess;
+}
+
 // the host-pointer path over all streams, or (n_rows > 0) over the compact rows a subset call gathered
 static int run_host(crispy_ns_batch *b, const void *h_in, void *h_out, float *h_vad, const float *h_app, int n_frames,
                     int64_t in_stride, int64_t out_stride, int64_t vad_stride, int64_t app_stride, uint32_t flags,
@@ -1097,44 +1073,10 @@ static int run_host(crispy_ns_batch *b, const void *h_in, void *h_out, float *h_
   const size_t in_bytes = (size_t)n * ch * ns::kFrame * ie, out_bytes = (size_t)n * ch * ns::kFrame * oe;
   const bool use_app = (flags & CRISPY_NS_MIX_STEREO_I16) && h_app;
   // (re)allocate double buffers
-  if (b->cap_in < in_bytes) {
-    for (int i = 0; i < 2; i++) {
-      if (b->d_in[i]) cudaFree(b->d_in[i]);
-      b->d_in[i] = nullptr;
-    }
-    NS_CUDA(cudaMalloc(&b->d_in[0], in_bytes));
-    NS_CUDA(cudaMalloc(&b->d_in[1], in_bytes));
-    b->cap_in = in_bytes;
-  }
-  if (b->cap_out < out_bytes) {
-    for (int i = 0; i < 2; i++) {
-      if (b->d_out[i]) cudaFree(b->d_out[i]);
-      b->d_out[i] = nullptr;
-    }
-    NS_CUDA(cudaMalloc(&b->d_out[0], out_bytes));
-    NS_CUDA(cudaMalloc(&b->d_out[1], out_bytes));
-    b->cap_out = out_bytes;
-  }
-  const size_t vad_bytes = (size_t)n * ch * sizeof(float);
-  if (h_vad && b->cap_vad < vad_bytes) {
-    for (int i = 0; i < 2; i++) {
-      if (b->d_vad[i]) cudaFree(b->d_vad[i]);
-      b->d_vad[i] = nullptr;
-    }
-    NS_CUDA(cudaMalloc((void **)&b->d_vad[0], vad_bytes));
-    NS_CUDA(cudaMalloc((void **)&b->d_vad[1], vad_bytes));
-    b->cap_vad = vad_bytes;
-  }
-  const size_t app_bytes = (size_t)n * ch * ns::kFrame * sizeof(float);
-  if (use_app && b->cap_app < app_bytes) {
-    for (int i = 0; i < 2; i++) {
-      if (b->d_app[i]) cudaFree(b->d_app[i]);
-      b->d_app[i] = nullptr;
-    }
-    NS_CUDA(cudaMalloc((void **)&b->d_app[0], app_bytes));
-    NS_CUDA(cudaMalloc((void **)&b->d_app[1], app_bytes));
-    b->cap_app = app_bytes;
-  }
+  NS_CUDA(fit_pair(b->d_in, b->cap_in, in_bytes));
+  NS_CUDA(fit_pair(b->d_out, b->cap_out, out_bytes));
+  if (h_vad) NS_CUDA(fit_pair(b->d_vad, b->cap_vad, (size_t)n * ch * sizeof(float)));
+  if (use_app) NS_CUDA(fit_pair(b->d_app, b->cap_app, (size_t)n * ch * ns::kFrame * sizeof(float)));
   const bool drop = (flags & CRISPY_NS_DROP_FIRST_FRAME) && b->frames_done == 0;
   int c = 0;
   for (long long f0 = 0; f0 < n_frames; f0 += ch, c++) {
@@ -1559,31 +1501,10 @@ int create(const crispy_ns_model *model, int device, crispy_ns_state **out) {
 // one frame of the state's single stream as a captured graph on st->s (built on the first use of each slot)
 static int frame_graph(crispy_ns_state *st, int slot) {
   crispy_ns_batch *b = st->b;
-  ns::Params p;
-  memset(&p, 0, sizeof(p));
-  p.in = st->d_io;
-  p.out = st->d_io + 480;
-  p.vad = st->d_io + 960;
-  p.state = b->d_state;
-  p.tables = b->d_tables;
-  p.rnn_hdr = b->d_hdr;
-  p.rnn_words = b->d_words;
-  p.rnn_bias = b->d_bias;
-  p.in_stride = 480;
-  p.out_stride = 480;
-  p.vad_stride = 1;
-  p.hp_stride = ns::kHist + (long long)b->chunk_cap * ns::kFrame;
-  p.n_streams = 1;
-  p.n_frames_call = 1;
-  p.n_frames = 1;
-  p.chunk_cap = b->chunk_cap;
-  p.volume = 1.0f;
-  p.hp = b->d_hp[slot];
-  p.tab = b->d_tab[slot];
-  p.rec = b->d_rec[slot];
-  p.spec = b->d_spec[slot];
-  p.featq = b->d_featq[slot];
-  p.synth_sel = slot & 1;  // == chunk counter & 1: kSlots is even
+  ns::Params p = ns::call_params(st->d_io, st->d_io + 480, st->d_io + 960, nullptr, nullptr, b->d_state, b->d_tables,
+                                 b->d_hdr, b->d_words, b->d_bias, 480, 480, 1, 0, 1, 1, b->chunk_cap, 0, 0, 1.0f);
+  // synth_sel == chunk counter & 1: kSlots is even
+  ns::set_chunk(p, 0, 1, b->d_hp[slot], b->d_tab[slot], b->d_rec[slot], b->d_spec[slot], b->d_featq[slot], slot & 1);
   static_assert(kSlots % 2 == 0, "the synthesis_mem parity follows the slot");
   NS_CUDA(cudaStreamBeginCapture(st->s, cudaStreamCaptureModeThreadLocal));
   cudaMemcpyAsync(st->d_io, st->h_pin, ns::kFrame * sizeof(float), cudaMemcpyHostToDevice, st->s);

@@ -235,4 +235,47 @@ struct Params {
   float volume;
 };
 
+// Host only: the Params of a call, every field but those of one chunk (set_chunk) and syn_run, which each caller picks
+inline Params call_params(const void *in, void *out, float *vad, const float *app, float *dbg, float *state,
+                          const Tables *tables, const RnnHeader *rnn_hdr, const uint32_t *rnn_words, const float *rnn_bias,
+                          long long in_stride, long long out_stride, long long vad_stride, long long app_stride,
+                          int n_streams, int n_frames_call, int chunk_cap, int out_frame_offset, uint32_t flags,
+                          float volume) {
+  Params p{};
+  p.in = in;
+  p.out = out;
+  p.vad = vad;
+  p.app = app;
+  p.dbg = dbg;
+  p.state = state;
+  p.tables = tables;
+  p.rnn_hdr = rnn_hdr;
+  p.rnn_words = rnn_words;
+  p.rnn_bias = rnn_bias;
+  p.in_stride = in_stride;
+  p.out_stride = out_stride;
+  p.vad_stride = vad_stride;
+  p.app_stride = app_stride;
+  p.hp_stride = kHist + (long long)chunk_cap * kFrame;
+  p.n_streams = n_streams;
+  p.n_frames_call = n_frames_call;
+  p.chunk_cap = chunk_cap;
+  p.out_frame_offset = out_frame_offset;
+  p.flags = flags;
+  p.volume = volume;
+  return p;
+}
+// Host only: the chunk of n_frames frames from frame0 of the call, in the workspace slot hp .. featq
+inline void set_chunk(Params &p, int frame0, int n_frames, float *hp, uint32_t *tab, float *rec, cf *spec,
+                      uint32_t *featq, int synth_sel) {
+  p.frame0 = frame0;
+  p.n_frames = n_frames;
+  p.hp = hp;
+  p.tab = tab;
+  p.rec = rec;
+  p.spec = spec;
+  p.featq = featq;
+  p.synth_sel = synth_sel;
+}
+
 }  // namespace ns

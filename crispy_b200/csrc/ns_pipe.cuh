@@ -24,6 +24,8 @@
 //
 // The same source compiles for sm_100a (nvcc) and for the host SIMT emulation (NS_HOST_EMU, tests).
 #pragma once
+#include <type_traits>
+
 #include "ns_common.h"
 #include "ns_simt.h"
 
@@ -2883,6 +2885,30 @@ inline int pick_syn_run(int n_streams, int n_frames, int resident_ctas) {
     }
   }
   return best;
+}
+
+// The kernel forms a model's numerics select (crispy_ns_model_set_numerics; host only).  K1 is instantiated per sum
+// order (pitch_body<R, NT, SP>), K0's single recursion warp per biquad arithmetic (highpass_body<F32>).  K0's
+// time-parallel form speculates the f64 expression only, so under kBiquadF32 the single recursion warp runs.
+constexpr uint32_t kSumMask = 3u, kBiquadF32 = 1u << 4;  // CRISPY_NS_SUM_MASK, CRISPY_NS_BIQUAD_F32
+#ifndef NS_PITCH_V7
+constexpr int kSumOrders = 3;
+#else
+constexpr int kSumOrders = 1;  // ns_pitch7.cuh sums in the sequential order only
+#endif
+inline bool numerics_valid(uint32_t numerics) {  // known bits, and sum order 3 is none
+  return !(numerics & ~(kSumMask | kBiquadF32)) && (numerics & kSumMask) != kSumMask;
+}
+inline bool biquad_f32(uint32_t numerics) { return (numerics & kBiquadF32) != 0; }
+inline bool hp_par_form(uint32_t numerics, bool par) { return par && !biquad_f32(numerics); }
+// f(std::integral_constant<int, SP>()) for the sum order of numerics; orders this build does not have run as 0
+template <class F>
+inline auto with_sum_order(uint32_t numerics, F &&f) {
+  if constexpr (kSumOrders > 1) {
+    if ((numerics & kSumMask) == 1) return f(std::integral_constant<int, 1>());
+    if ((numerics & kSumMask) == 2) return f(std::integral_constant<int, 2>());
+  }
+  return f(std::integral_constant<int, 0>());
 }
 
 // one thread stages a frame's spectra (X | P, 7,712 B) and record (592 B) into buffer b: two bulk copies on s.mbar

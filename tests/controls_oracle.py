@@ -12,19 +12,13 @@ Nothing else of the oracle changes, and the build refuses to proceed if the sour
 """
 from __future__ import annotations
 
-import atexit
 import ctypes as C
-import os
-import shutil
-import subprocess
-import tempfile
 
 import numpy as np
 
 from oracle import pyoracle as po
+from tests.util import patched_oracle
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-SRC = os.path.join(ROOT, "oracle", "rnnoise_oracle.c")
 INCLUDE = "#include <string.h>\n"
 APPLY = "    interp_band_gain(gf, g);\n"
 APPLY_FLOORED = """    if (g_ctl_min_gain > 0.f) {
@@ -84,18 +78,7 @@ def lib() -> C.CDLL:
     """the oracle with the controls (pyoracle's bindings, plus rno_controls_*)"""
     global _lib
     if _lib is None:
-        src = open(SRC).read()
-        assert src.count(INCLUDE) == 1 and src.count(APPLY) == 1 and src.count(AUDIBLE) == 1, \
-            "the oracle's gain application changed: update tests/controls_oracle.py"
-        src = (src.replace(INCLUDE, INCLUDE + GLOBAL).replace(APPLY, APPLY_FLOORED).replace(AUDIBLE, AUDIBLE_FLOORED)
-               + ENTRY)
-        d = tempfile.mkdtemp(prefix="crispy_oracle_controls_")
-        atexit.register(shutil.rmtree, d, True)
-        c_path, so_path = os.path.join(d, "rnnoise_oracle_controls.c"), os.path.join(d, "librnnoise_oracle_controls.so")
-        open(c_path, "w").write(src)
-        subprocess.check_call(["gcc", "-O2", "-fPIC", "-ffp-contract=off", "-fno-fast-math", "-std=c11", "-shared",
-                               "-I" + os.path.join(ROOT, "oracle"), "-o", so_path, c_path, "-lm", "-lpthread"])
-        L = po._declare(C.CDLL(so_path))
+        L = patched_oracle([(INCLUDE, INCLUDE + GLOBAL), (APPLY, APPLY_FLOORED), (AUDIBLE, AUDIBLE_FLOORED)], ENTRY)
         f32p = C.POINTER(C.c_float)
         L.rno_controls_process_frame.argtypes = [C.c_void_p, C.POINTER(Controls), f32p, f32p]
         L.rno_controls_process_frame.restype = C.c_float

@@ -91,11 +91,13 @@ int ns_emu_hp_spec(void) { return NS_HP_PAR; }
 long long ns_emu_hp_respeculated(void) { return __atomic_exchange_n(&ns::g_hp_respeculated, 0, __ATOMIC_RELAXED); }
 
 // in/out/app use the same strides the device path uses; state is in/out ([n_streams][kStateFloats]).
-// The call is cut into chunks of `chunk_cap` frames exactly as libcrispy_ns.so does.
+// The call is cut into chunks of `chunk_cap` frames exactly as libcrispy_ns.so does.  numerics: the model's setting
+// (crispy_ns_model_set_numerics); -3 for one the library refuses, a nonzero sum order in the NS_PITCH_V7 build included.
 int ns_emu_process(const void *model_blob, size_t model_len, const void *in, void *out, float *vad,
                    const float *app, float *state, float *dbg, int n_streams, int n_frames,
                    long long in_stride, long long out_stride, long long app_stride, int chunk_cap,
-                   unsigned flags, float volume, int out_frame_offset) {
+                   unsigned flags, float volume, int out_frame_offset, unsigned numerics) {
+  if (!ns::numerics_valid(numerics) || (int)(numerics & ns::kSumMask) >= ns::kSumOrders) return -3;
   ns::Model m;
   std::string err;
   if (!ns::model_from_bytes(m, model_blob, model_len, err)) {
@@ -107,65 +109,44 @@ int ns_emu_process(const void *model_blob, size_t model_len, const void *in, voi
   static ns::Tables tab;
   ns::make_tables(tab);
   if (chunk_cap < 1) chunk_cap = 8;
-  ns::Params p;
-  memset(&p, 0, sizeof(p));
-  const long long hp_stride = ns::kHist + (long long)chunk_cap * ns::kFrame;
-  std::vector<float> hp((size_t)n_streams * hp_stride, 0.f);
+  ns::Params p = ns::call_params(in, out, vad, app, dbg, state, &tab, &pk.hdr, pk.words.data(), pk.bias.data(), in_stride,
+                                 out_stride, n_frames, app_stride, n_streams, n_frames, chunk_cap, out_frame_offset, flags,
+                                 volume);
+  std::vector<float> hp((size_t)n_streams * p.hp_stride, 0.f);
   std::vector<uint32_t> tabw((size_t)n_streams * chunk_cap * ns::kTabWords, 0u);
   std::vector<float> rec((size_t)n_streams * chunk_cap * ns::kRecFloats, 0.f);
   std::vector<ns::cf> spec((size_t)n_streams * chunk_cap * 2 * ns::kSpecStride);
   const int groups = (n_streams + ns::kMmaStreams - 1) / ns::kMmaStreams;
   std::vector<uint32_t> featq((size_t)groups * chunk_cap * ns::kFeatBlockWords, 0xCDCDCDCDu);
-  p.in = in;
-  p.out = out;
-  p.vad = vad;
-  p.app = app;
-  p.dbg = dbg;
-  p.state = state;
-  p.hp = hp.data();
-  p.tab = tabw.data();
-  p.rec = rec.data();
-  p.spec = spec.data();
-  p.featq = featq.data();
-  p.tables = &tab;
-  p.rnn_hdr = &pk.hdr;
-  p.rnn_words = pk.words.data();
-  p.rnn_bias = pk.bias.data();
-  p.in_stride = in_stride;
-  p.out_stride = out_stride;
-  p.vad_stride = n_frames;
-  p.app_stride = app_stride;
-  p.hp_stride = hp_stride;
-  p.n_streams = n_streams;
-  p.n_frames_call = n_frames;
-  p.chunk_cap = chunk_cap;
-  p.out_frame_offset = out_frame_offset;
-  p.flags = flags;
-  p.volume = volume;
+  // both forms of K0 (the library picks by batch size; here $CRISPY_NS_HP_PAR = 0 selects the single recursion warp)
+  const char *hpp = getenv("CRISPY_NS_HP_PAR");
+  const bool hp_par = ns::hp_par_form(numerics, hpp ? atoi(hpp) != 0 : NS_HP_PAR != 0);
+  const bool f32 = ns::biquad_f32(numerics);
   for (int f0 = 0; f0 < n_frames; f0 += chunk_cap) {
     const int nf = (n_frames - f0) < chunk_cap ? (n_frames - f0) : chunk_cap;
-    p.frame0 = f0;
-    p.n_frames = nf;
     // the library keeps its chunk counter in the batch handle; the emulation keeps it in stream 0's
     // state block (host side) so that chained calls see the same synthesis_mem buffer parity
     int *chunk_counter = reinterpret_cast<int *>(state) + ns::kStateFloats - 1;
-    p.synth_sel = *chunk_counter & 1;
+    ns::set_chunk(p, f0, nf, hp.data(), tabw.data(), rec.data(), spec.data(), featq.data(), *chunk_counter & 1);
     *chunk_counter += 1;
-    // both forms of K0 (the library picks by batch size; here $CRISPY_NS_HP_PAR = 0 selects the single recursion warp)
-    const char *hpp = getenv("CRISPY_NS_HP_PAR");
-    const bool hp_par = hpp ? atoi(hpp) != 0 : NS_HP_PAR != 0;
     int rc = hp_par ? launch((n_streams + 31) / 32, ns::kHpParThreads, sizeof(ns::HpParSmem),
                              [&](void *sm) { ns::highpass_par_body(p, *(ns::HpParSmem *)sm); })
-                    : launch((n_streams + 31) / 32, ns::kHpThreads, sizeof(ns::HpSmem),
-                             [&](void *sm) { ns::highpass_body(p, *(ns::HpSmem *)sm); });
+                    : launch((n_streams + 31) / 32, ns::kHpThreads, sizeof(ns::HpSmem), [&](void *sm) {
+                        if (f32)
+                          ns::highpass_body<true>(p, *(ns::HpSmem *)sm);
+                        else
+                          ns::highpass_body<false>(p, *(ns::HpSmem *)sm);
+                      });
     if (rc) return rc;
     const int runs = (nf + kPitchRun - 1) / kPitchRun;
     rc = launch(n_streams * runs, kPitchThreads, sizeof(PitchShared), [&](void *sm) {
+      ns::with_sum_order(numerics, [&](auto sp) {
 #ifndef NS_PITCH_V7
-      ns::pitch_body<kPitchRun, kPitchThreads>(p, *(PitchShared *)sm);
+        ns::pitch_body<kPitchRun, kPitchThreads, decltype(sp)::value>(p, *(PitchShared *)sm);
 #else
-      ns::pitch_body7<kPitchRun, kPitchThreads>(p, *(PitchShared *)sm);
+        ns::pitch_body7<kPitchRun, kPitchThreads>(p, *(PitchShared *)sm);
 #endif
+      });
     });
     if (rc) return rc;
     rc = launch((n_streams + kScanWarps - 1) / kScanWarps, 32 * kScanWarps, 16,
@@ -187,5 +168,15 @@ int ns_emu_process(const void *model_blob, size_t model_len, const void *in, voi
     if (rc) return rc;
   }
   return 0;
+}
+
+// the per-stream suppression controls (crispy_ns_controls) on row `stream` of a state as ns_emu_process takes it, word
+// for word as libcrispy_ns.so's ns_set_controls_kernel writes them; the gate's carry is left alone
+void ns_emu_set_controls(float *state, int stream, float min_gain, float gate_threshold, int gate_hold, float gate_gain) {
+  float *row = state + (size_t)stream * ns::kStateFloats;
+  row[ns::kStCtlMinGain] = min_gain;
+  row[ns::kStCtlGateThr] = gate_threshold;
+  memcpy(&row[ns::kStCtlGateHold], &gate_hold, 4);
+  row[ns::kStCtlGateGain] = gate_gain;
 }
 }

@@ -11,19 +11,13 @@ the oracle changes, and the build refuses to proceed if the source no longer has
 """
 from __future__ import annotations
 
-import atexit
 import ctypes as C
-import os
-import shutil
-import subprocess
-import tempfile
 
 import numpy as np
 
 from oracle import pyoracle as po
+from tests.util import patched_oracle
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-SRC = os.path.join(ROOT, "oracle", "rnnoise_oracle.c")
 CALL = "biquad(x, st->mem_hp_x, in, b_hp, a_hp, FRAME_SIZE);"
 DEF = "static void biquad(float *y, float mem[2], const float *x, const float *b, const float *a, int N) {"
 F32_BIQUAD = """static void biquad_f32(float *y, float mem[2], const float *x, const float *b, const float *a, int N) {
@@ -52,16 +46,7 @@ def lib_f32() -> C.CDLL:
     """the oracle with the f32 biquad (pyoracle's bindings, plus rno_numerics_highpass_f32)"""
     global _lib
     if _lib is None:
-        src = open(SRC).read()
-        assert src.count(CALL) == 1 and src.count(DEF) == 1, "the oracle's biquad call changed: update tests/numerics_oracle.py"
-        src = src.replace(DEF, F32_BIQUAD + DEF).replace(CALL, "biquad_f32" + CALL[len("biquad"):]) + HIGHPASS
-        d = tempfile.mkdtemp(prefix="crispy_oracle_f32_")
-        atexit.register(shutil.rmtree, d, True)
-        c_path, so_path = os.path.join(d, "rnnoise_oracle_f32.c"), os.path.join(d, "librnnoise_oracle_f32.so")
-        open(c_path, "w").write(src)
-        subprocess.check_call(["gcc", "-O2", "-fPIC", "-ffp-contract=off", "-fno-fast-math", "-std=c11", "-shared",
-                               "-I" + os.path.join(ROOT, "oracle"), "-o", so_path, c_path, "-lm", "-lpthread"])
-        L = po._declare(C.CDLL(so_path))
+        L = patched_oracle([(DEF, F32_BIQUAD + DEF), (CALL, "biquad_f32" + CALL[len("biquad"):])], HIGHPASS)
         f32p = C.POINTER(C.c_float)
         L.rno_numerics_highpass_f32.argtypes = [f32p, f32p, f32p, C.c_int]
         L.rno_numerics_highpass_f32.restype = None

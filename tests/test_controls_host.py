@@ -1,14 +1,11 @@
 """CPU: the per-stream suppression controls (crispy_ns_controls: attenuation limit and voice gate).  The C boundary's
 contract without a device, the oracle under the controls (tests/controls_oracle.py) against a NumPy float32
 transliteration of the gate (tests/controls_ref.py), and K4 / K5 under the host SIMT emulation
-(tests/emu/ns_emu_controls.cpp) with different controls per stream against that oracle under the same controls."""
-import atexit
+(tests/emu/ns_emu.cpp) with different controls per stream against that oracle under the same controls."""
 import ctypes as C
 import os
 import re
-import shutil
 import subprocess
-import tempfile
 
 import numpy as np
 import pytest
@@ -18,7 +15,7 @@ from crispy_b200 import _lib, build
 from oracle import pyoracle as po
 from tests import controls_oracle as co
 from tests import controls_ref as cr
-from tests.util import BRANCH_EPS, CSRC, EMU_DIR, TOL_MAX_ABS, TOL_SNR_DB, TOL_VAD, make_signal, snr_db
+from tests.util import BRANCH_EPS, TOL_MAX_ABS, TOL_SNR_DB, TOL_VAD, emu_lib, emu_process, make_signal, snr_db
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 EINVAL, ENODEV = -1, -2
@@ -174,44 +171,12 @@ def test_gate_and_floor_are_not_vacuous(oracle_off, oracle_on):
 
 
 # ---- K4 / K5 under the host emulation --------------------------------------------------------------------------------
-_emu = None
-
-
-def emu_lib():
-    """tests/emu/ns_emu_controls.cpp, built once per process into a temporary directory"""
-    global _emu
-    if _emu is None:
-        d = tempfile.mkdtemp(prefix="crispy_emu_controls_")
-        atexit.register(shutil.rmtree, d, True)
-        so = os.path.join(d, "libns_emu_controls.so")
-        subprocess.check_call(["g++", "-O2", "-std=c++17", "-fPIC", "-shared", "-pthread", "-ffp-contract=off",
-                               "-Wno-unknown-pragmas", "-o", so, os.path.join(EMU_DIR, "ns_emu_controls.cpp"),
-                               os.path.join(CSRC, "ns_host.cpp")])
-        L = C.CDLL(so)
-        L.ns_emu_process.argtypes = [C.c_char_p, C.c_size_t, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
-                                     C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_longlong, C.c_longlong,
-                                     C.c_longlong, C.c_int, C.c_uint, C.c_float, C.c_int]
-        L.ns_emu_set_controls.argtypes = [C.c_void_p, C.c_int, C.c_float, C.c_float, C.c_int, C.c_float]
-        L.ns_emu_set_controls.restype = None
-        _emu = L
-    return _emu
-
-
 def emu_run(blob, x, controls, chunk=CHUNK):
     L = emu_lib()
-    x = np.ascontiguousarray(x, dtype=np.float32)
-    ns, n = x.shape
-    nf = n // 480
-    out = np.zeros_like(x)
-    vad = np.zeros((ns, nf), np.float32)
-    dbg = np.zeros((ns, nf, L.ns_emu_dbg_floats()), np.float32)
-    state = np.zeros((ns, L.ns_emu_state_floats()), np.float32)
+    state = np.zeros((x.shape[0], L.ns_emu_state_floats()), np.float32)
     for s, c in enumerate(controls):
         L.ns_emu_set_controls(state.ctypes.data, s, *c)
-    rc = L.ns_emu_process(blob, len(blob), x.ctypes.data, out.ctypes.data, vad.ctypes.data, None, state.ctypes.data,
-                          dbg.ctypes.data, ns, nf, n, n, 0, chunk, 0, 1.0, 0)
-    assert rc == 0, rc
-    return out, vad, dbg, state
+    return emu_process(blob, x, chunk=chunk, state=state)
 
 
 @pytest.fixture(scope="module")

@@ -1,14 +1,11 @@
 """CPU: the model's numerics setting (crispy_ns_model_set_numerics) at the C boundary, the oracle's f32 biquad
 (tests/numerics_oracle.py), and the pitch and biquad kernels under every combination of sum order and biquad form, run
-under the host SIMT emulation (tests/emu/ns_emu_numerics.cpp) against the oracle under the same combination."""
-import atexit
+under the host SIMT emulation (tests/emu/ns_emu.cpp) against the oracle under the same combination."""
 import ctypes as C
 import itertools
 import os
 import re
-import shutil
 import subprocess
-import tempfile
 
 import numpy as np
 import pytest
@@ -16,7 +13,7 @@ import pytest
 import crispy_b200 as cb
 from crispy_b200 import _lib, build
 from tests import numerics_oracle as no
-from tests.util import CSRC, EMU_DIR, assert_parity, make_signal
+from tests.util import assert_parity, emu_lib, emu_process, make_signal
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 EINVAL, ENODEV = -1, -2
@@ -144,42 +141,6 @@ def test_oracle_f32_biquad_is_the_float32_transliteration_and_not_the_f64_form()
 
 
 # ---- the kernels under the host emulation ----------------------------------------------------------------------------
-_emu = None
-
-
-def emu_lib():
-    """tests/emu/ns_emu_numerics.cpp (the emulation of tests/emu/ns_emu.cpp plus a numerics entry point), built once per
-    process into a temporary directory"""
-    global _emu
-    if _emu is None:
-        d = tempfile.mkdtemp(prefix="crispy_emu_numerics_")
-        atexit.register(shutil.rmtree, d, True)
-        so = os.path.join(d, "libns_emu_numerics.so")
-        subprocess.check_call(["g++", "-O2", "-std=c++17", "-fPIC", "-shared", "-pthread", "-ffp-contract=off",
-                               "-Wno-unknown-pragmas", "-o", so, os.path.join(EMU_DIR, "ns_emu_numerics.cpp"),
-                               os.path.join(CSRC, "ns_host.cpp")])
-        _emu = C.CDLL(so)
-    return _emu
-
-
-def emu_run(blob, x, numerics, chunk=8):
-    L = emu_lib()
-    L.ns_emu_process_numerics.argtypes = [C.c_char_p, C.c_size_t, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
-                                          C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_longlong, C.c_longlong,
-                                          C.c_longlong, C.c_int, C.c_uint, C.c_float, C.c_int, C.c_uint]
-    x = np.ascontiguousarray(x, dtype=np.float32)
-    ns, n = x.shape
-    nf = n // 480
-    out = np.zeros_like(x)
-    vad = np.zeros((ns, nf), np.float32)
-    dbg = np.zeros((ns, nf, L.ns_emu_dbg_floats()), np.float32)
-    state = np.zeros((ns, L.ns_emu_state_floats()), np.float32)
-    rc = L.ns_emu_process_numerics(blob, len(blob), x.ctypes.data, out.ctypes.data, vad.ctypes.data, None,
-                                   state.ctypes.data, dbg.ctypes.data, ns, nf, n, n, 0, chunk, 0, 1.0, 0, numerics)
-    assert rc == 0, rc
-    return out, vad, dbg, state
-
-
 @pytest.fixture(scope="module")
 def sig():
     return make_signal(3, 28)
@@ -192,7 +153,7 @@ def oracle_runs(model_blob, sig):
 
 @pytest.fixture(scope="module")
 def emu_runs(model_blob, sig):
-    return {nm: emu_run(model_blob, sig, nm) for nm in COMBOS}
+    return {nm: emu_process(model_blob, sig, chunk=8, numerics=nm) for nm in COMBOS}
 
 
 @pytest.mark.parametrize("numerics", COMBOS)
@@ -208,7 +169,6 @@ def test_emulated_kernels_match_the_oracle_under_the_same_numerics(oracle_runs, 
 
 
 def test_numerics_zero_entry_point_is_the_existing_one(model_blob, sig, emu_runs):
-    from tests.util import emu_process
     out, vad, dbg, st = emu_process(model_blob, sig, chunk=8)
     o0, v0, d0, s0 = emu_runs[0]
     assert np.array_equal(out, o0) and np.array_equal(vad, v0) and np.array_equal(dbg, d0) and np.array_equal(st, s0)
@@ -234,7 +194,7 @@ def test_the_switches_are_not_vacuous(oracle_runs, emu_runs):
 def test_emulated_f32_biquad_is_the_float32_transliteration(model_blob):
     x = (2500.0 * np.random.default_rng(4).standard_normal((2, 4 * 480))).astype(np.float32)
     hp = emu_lib().ns_emu_state_hp_offset()
-    _, _, _, st = emu_run(model_blob, x, _lib.BIQUAD_F32, chunk=3)
+    _, _, _, st = emu_process(model_blob, x, chunk=3, numerics=_lib.BIQUAD_F32)
     for s in range(2):
         y, m0, m1 = _biquad_f32_numpy(x[s])
         assert st[s, hp:hp + 2].view(np.uint32).tolist() == [np.float32(m0).view(np.uint32), np.float32(m1).view(np.uint32)]

@@ -1,11 +1,16 @@
 """Shared helpers for the test-suite (test plumbing only)."""
 from __future__ import annotations
 
+import atexit
 import ctypes as C
 import os
+import shutil
 import subprocess
+import tempfile
 
 import numpy as np
+
+from oracle import pyoracle as po
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 EMU_DIR = os.path.join(ROOT, "tests", "emu")
@@ -38,14 +43,19 @@ def emu_lib(v7: bool = False):
         L = C.CDLL(build_emu(v7))
         L.ns_emu_process.argtypes = [C.c_char_p, C.c_size_t, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                      C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_longlong, C.c_longlong,
-                                     C.c_longlong, C.c_int, C.c_uint, C.c_float, C.c_int]
+                                     C.c_longlong, C.c_int, C.c_uint, C.c_float, C.c_int, C.c_uint]
+        L.ns_emu_set_controls.argtypes = [C.c_void_p, C.c_int, C.c_float, C.c_float, C.c_int, C.c_float]
+        L.ns_emu_set_controls.restype = None
+        L.ns_emu_hp_respeculated.restype = C.c_longlong
         _emu[v7] = L
     return _emu[v7]
 
 
 def emu_process(blob: bytes, x: np.ndarray, chunk: int = 16, flags: int = 0, volume: float = 1.0, state=None,
-                out_dtype=np.float32, out_cols=None, app=None, out_frame_offset: int = 0, v7: bool = False):
-    """Run the kernel body under the host SIMT emulation.  x: [n_streams, n_frames*480]."""
+                out_dtype=np.float32, out_cols=None, app=None, out_frame_offset: int = 0, v7: bool = False,
+                numerics: int = 0):
+    """Run the kernel body under the host SIMT emulation.  x: [n_streams, n_frames*480]; numerics: the model's setting
+    (crispy_ns_model_set_numerics)."""
     L = emu_lib(v7)
     x = np.ascontiguousarray(x)
     ns, n = x.shape
@@ -62,9 +72,28 @@ def emu_process(blob: bytes, x: np.ndarray, chunk: int = 16, flags: int = 0, vol
     out_stride = out.shape[1] if not (flags & 8) else out.shape[1] // 2
     rc = L.ns_emu_process(blob, len(blob), x.ctypes.data, out.ctypes.data, vad.ctypes.data, app_p,
                           state.ctypes.data, dbg.ctypes.data, ns, nf, n, out_stride, app_stride, chunk, flags,
-                          volume, out_frame_offset)
+                          volume, out_frame_offset, numerics)
     assert rc == 0, f"ns_emu_process failed: {rc}"
     return out, vad, dbg, state
+
+
+def patched_oracle(edits, appended: str) -> C.CDLL:
+    """oracle/rnnoise_oracle.c with each (old, new) of `edits` made and `appended` added at its end, compiled as the
+    oracle's own build is into a temporary directory of this process (removed at exit), with pyoracle's bindings
+    declared.  Each `old` must occur exactly once in the source, so that a changed oracle stops the build."""
+    src = open(os.path.join(ROOT, "oracle", "rnnoise_oracle.c")).read()
+    for old, _ in edits:
+        assert src.count(old) == 1, f"the oracle no longer has exactly one {old!r}: update the patch"
+    for old, new in edits:
+        src = src.replace(old, new)
+    d = tempfile.mkdtemp(prefix="crispy_oracle_patched_")
+    atexit.register(shutil.rmtree, d, True)
+    c_path, so_path = os.path.join(d, "rnnoise_oracle.c"), os.path.join(d, "librnnoise_oracle.so")
+    with open(c_path, "w") as f:
+        f.write(src + appended)
+    subprocess.check_call(["gcc", "-O2", "-fPIC", "-ffp-contract=off", "-fno-fast-math", "-std=c11", "-shared",
+                           "-I" + os.path.join(ROOT, "oracle"), "-o", so_path, c_path, "-lm", "-lpthread"])
+    return po._declare(C.CDLL(so_path))
 
 
 def snr_db(ref: np.ndarray, test: np.ndarray) -> float:
